@@ -12,10 +12,12 @@ action (actor resolution -> observation -> reward/done); the K timed steps are e
 (= K x bgw_step_sampled; on the specialised kernel one launch whose CTAs draw (step, env) tickets).  An agent-step = one
 learning agent receiving (obs, reward, done).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  With --dump-outputs, rank 0 also writes what the last timed step returned (see
+dump_outputs): the inputs depend on the arguments alone, so two builds run with the same arguments can be compared output
+for output.
 """
 import argparse
 import json
@@ -88,6 +90,26 @@ class ClockSampler(threading.Thread):
         reasons = sorted({n for r in rows for n, v in zip(names, r[5:9]) if v.lower().startswith('active')})
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": reasons, "samples": len(sm), "period_ms": 50}
+
+
+DUMP_ENVS = 256                 # envs of the --dump-outputs sample: obs of 256 envs x 256 learners x 11x11 in float32 = 32 MB
+
+
+def dump_outputs(eng, out_dir, n_envs=DUMP_ENVS):
+    """Write to `out_dir`/<name>.npy what the caller of the timed path receives after its last step -- obs (the logical
+    [h, w] view of the padded rows), reward, done, all_done and the sampled actions -- for a fixed, seeded sample of
+    `n_envs` envs (all envs if there are fewer; their indices in env_index.npy), and the episode statistics summed over all
+    envs (stats.npy: agent_steps, episodes, kills, env_steps).  float32, or float64 where float32 would round."""
+    import torch
+    envs = np.sort(np.random.default_rng(0xB200).choice(eng.E, size=min(eng.E, n_envs), replace=False))
+    idx = torch.from_numpy(envs).to(eng.device)
+    pick = lambda t: t.index_select(0, idx).cpu().numpy().astype(np.float32)
+    arrays = {'env_index': envs.astype(np.float64), 'obs': pick(eng.obs_view()), 'reward': pick(eng.reward),
+              'done': pick(eng.done), 'all_done': pick(eng.all_done), 'actions': pick(eng.actions),
+              'stats': eng.stats().cpu().numpy().astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def measured_peak():
@@ -225,6 +247,8 @@ def run_ours(args):
     ms = t_beg.elapsed_time(t_end)
     n_dev = agent_steps() - n0
     launches = eng.launches - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, args.dump_outputs)
     kernel_ms = ms
     ks = max(1, min(args.kernel_steps, args.steps))
     k_ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(ks)]
@@ -452,6 +476,8 @@ def main():
     ap.add_argument('--e2e-zero-copy', action='store_true', help='e2e: the gather kernel writes the pinned host buffers directly instead of compacting on the device and copying')
     ap.add_argument('--observe-launches', type=int, default=50, help='bgw_observe launches timed next to the step kernel')
     ap.add_argument('--dump-steps', default=None, help='write the per-step kernel times (ms) to this JSON file')
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                    help="write the outputs of the last timed step (rank 0's envs) to DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
     if args.impl == 'reference':
         run_reference(args)

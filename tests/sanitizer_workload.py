@@ -1,5 +1,6 @@
+import os
 import sys
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from tests import scenarios
 from abmarl_b200.spec import compile_sim
