@@ -512,6 +512,10 @@ int bgw_create(const BgwSpec *sp, int device, bgw_handle *out)
         h->observe_grid = std::max(1, std::min(d.E, per_sm * sms));
         if (const char *t = getenv("BGW_OBSERVE_GRID")) { const int v = atoi(t); if (v >= 1) h->observe_grid = std::min(d.E, v); }
     }
+    if (getenv("BGW_VERBOSE")) {
+        if (h->observe_fn) fprintf(stderr, "[bgw] observe kernel: gather-only, view %d\n", h->fs.uniform_view);
+        else fprintf(stderr, "[bgw] observe kernel: general\n");
+    }
     if (h->fs.enabled) {
         int per_sm = 0, sms = 0;
         /* the instantiation step_impl launches for this handle */

@@ -1339,6 +1339,9 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
 
         if (fresh) {
             for (int i = tid; i < n_act; i += T) ev.plist[i] = f.identity_learners ? ev.ragent[i] : (uint16_t)__ldg(&s.learner_of[ev.ragent[i]]);
+            /* the observation gather below reads entries other threads wrote (with every entity a learner, plist is ragent,
+             * which the compaction's barrier published) */
+            if (!f.identity_learners) __syncthreads();
         } else {
             /* ---- attack phase team_battle_example.py:35-47 ---------------------------------------------- */
             for (int i = tid; i < n_act; i += T) {
