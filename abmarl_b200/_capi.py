@@ -16,7 +16,7 @@ BGW_STAT_COUNT = 4
 # enums (include/bgw.h)
 AG_OBSERVING, AG_MOVING, AG_ATTACKING, AG_HEALTH, AG_ORIENT, AG_LEARNER, AG_BLOCKING, AG_AMMO = (1 << i for i in range(8))
 ROLE_NONE, ROLE_NAVIGATOR, ROLE_TARGET, ROLE_PACMAN, ROLE_FOOD, ROLE_BADDIE, ROLE_WALL, ROLE_RUNNER = range(8)
-PROG_TEAM_BATTLE, PROG_MAZE, PROG_MULTI_MAZE, PROG_PACMAN, PROG_REACH_TARGET, PROG_TRAFFIC, PROG_PACMAN_SIMPLE = range(7)
+PROG_TEAM_BATTLE, PROG_MAZE, PROG_MULTI_MAZE, PROG_PACMAN, PROG_REACH_TARGET, PROG_TRAFFIC, PROG_PACMAN_SIMPLE, PROG_USER = range(8)
 ROLE_SCRIPTED_BADDIE = 16
 MOVE_NONE, MOVE_BOX, MOVE_CROSS, MOVE_DRIFT = range(4)
 ATTACK_NONE, ATTACK_BINARY, ATTACK_ENCODING, ATTACK_RESTRICTED, ATTACK_SELECTIVE = range(5)
@@ -31,7 +31,7 @@ OUT_DONE, OUT_VALID = 1, 2
 ENV_ALL_DONE, ENV_RESET, ENV_TRUNCATED, ENV_ERROR = 1, 2, 4, 8
 STAT_AGENT_STEPS, STAT_EPISODES, STAT_KILLS, STAT_ENV_STEPS = range(4)
 SITE_PLACE, SITE_HEALTH, SITE_ORIENT, SITE_ACC, SITE_SUBSET, SITE_OBS, SITE_ACTION, SITE_MAZE, SITE_AMMO, SITE_SCRIPT, \
-    SITE_ORDER, SITE_PLACE_ORDER = range(12)
+    SITE_ORDER, SITE_PLACE_ORDER, SITE_PROGRAM = range(13)
 
 _p = C.c_void_p
 
@@ -67,7 +67,7 @@ class BgwDims(C.Structure):
 
 LAYOUT_POSITION_STATE, LAYOUT_MAZE, LAYOUT_TARGET_BARRIERS_FREE = range(3)
 
-EXPORTS = ('bgw_create', 'bgw_destroy', 'bgw_dims', 'bgw_bind_state', 'bgw_reset', 'bgw_observe', 'bgw_specialize', 'bgw_step', 'bgw_generate_layouts',
+EXPORTS = ('bgw_create', 'bgw_destroy', 'bgw_dims', 'bgw_bind_state', 'bgw_reset', 'bgw_observe', 'bgw_specialize', 'bgw_set_program', 'bgw_step', 'bgw_generate_layouts',
            'bgw_maze_layout_host', 'bgw_use_device_layouts',
            'bgw_sample_actions', 'bgw_step_sampled', 'bgw_rollout_sampled', 'bgw_gather_valid', 'bgw_rng_draw', 'bgw_los_mask', 'bgw_launch_count', 'bgw_last_error',
            'bgw_abi_version')
@@ -103,6 +103,8 @@ def load():
     lib.bgw_observe.restype = C.c_int
     lib.bgw_specialize.argtypes = [h, C.c_char_p]
     lib.bgw_specialize.restype = C.c_int
+    lib.bgw_set_program.argtypes = [h, C.c_char_p, C.c_char_p]
+    lib.bgw_set_program.restype = C.c_int
     lib.bgw_step_sampled.argtypes = [h, _p, _p, _p, _p, _p, _p, _p]
     lib.bgw_step_sampled.restype = C.c_int
     lib.bgw_rollout_sampled.argtypes = [h, C.c_int, _p, _p, _p, _p, _p, _p, _p]

@@ -23,7 +23,7 @@
 
 namespace {
 
-thread_local char g_err[512] = "";
+thread_local char g_err[2048] = "";   /* room for an NVRTC diagnostic (bgw_set_program) */
 
 int fail(int code, const char *fmt, ...)
 {
@@ -66,7 +66,7 @@ static const void *observe_fast_fn(int R)
 struct BgwEngine {
     int device = 0;
     GeneralStepFn step_fn = nullptr;   /* the bgw_step_kernel instantiation of this sim's program */
-    bgwjit::Kernel jit;                /* bgw_specialize: the same body compiled at run time for this spec alone (launched instead of step_fn) */
+    bgwjit::Kernel jit;                /* bgw_specialize / bgw_set_program: the same body compiled at run time for this spec alone (launched instead of step_fn) */
     bgwjit::Kernel fast_jit;           /* bgw_specialize: the specialised kernel's body with this spec's shape as its compile-time shape */
     bool fast_jit_on = false;          /* launch fast_jit instead of fast_fn (off again when the caller binds its own layouts) */
     const void *fast_fn = nullptr;     /* the bgw_step_fast_kernel instantiation of this sim's shape */
@@ -274,7 +274,9 @@ int bgw_create(const BgwSpec *sp, int device, bgw_handle *out)
         return bail(fail(1, "bgw_create: PacmanSim needs a learning pacman and the (9,0)<->(9,20) tunnel (pacman.py:87-92)"));
     if (sp->program == BGW_PROG_REACH_TARGET && (d.a_target < 0 || learner_of[d.a_target] < 0))
         return bail(fail(1, "bgw_create: ReachTheTargetSim needs a learning target agent"));
-    if (sp->program < BGW_PROG_TEAM_BATTLE || sp->program > BGW_PROG_PACMAN_SIMPLE) return bail(fail(1, "bgw_create: unknown program %d", sp->program));
+    if (sp->program < BGW_PROG_TEAM_BATTLE || sp->program > BGW_PROG_USER) return bail(fail(1, "bgw_create: unknown program %d", sp->program));
+    if (sp->program == BGW_PROG_USER && sp->manager == BGW_MANAGER_DYNAMIC_ORDER)
+        return bail(fail(1, "bgw_create: a user step program cannot run under BGW_MANAGER_DYNAMIC_ORDER (its next_agent rule is built in)"));
 
     /* ---- observation geometry (same rule as the oracle's bgwo_dims) ------------------------------ */
     BgwDims &dm = h->dims;
@@ -491,9 +493,10 @@ int bgw_create(const BgwSpec *sp, int device, bgw_handle *out)
     d.smem_bytes = off;
     if (off > 227 * 1024) return bail(fail(1, "bgw_create: one environment needs %d bytes of shared memory (limit 232448): grid or entity count too large", off));
     cudaError_t ce;
-    h->step_fn = bgw_general_step_fn(d.program, d.attack_actor);
-    if (const char *t = getenv("BGW_ALL_IN_ONE_KERNEL")) if (atoi(t)) h->step_fn = bgw_general_step_fn(-1, -1);
-    if ((ce = cudaFuncSetAttribute(h->step_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, off)) != cudaSuccess ||
+    /* a user step program has no stock instantiation: its kernel comes from bgw_set_program */
+    h->step_fn = d.program == BGW_PROG_USER ? nullptr : bgw_general_step_fn(d.program, d.attack_actor);
+    if (const char *t = getenv("BGW_ALL_IN_ONE_KERNEL")) if (atoi(t) && h->step_fn) h->step_fn = bgw_general_step_fn(-1, -1);
+    if ((h->step_fn && (ce = cudaFuncSetAttribute(h->step_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, off)) != cudaSuccess) ||
         (h->fs.enabled && (ce = cudaFuncSetAttribute(h->fast_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, h->fs.smem_bytes)) != cudaSuccess) ||
         (ce = cudaFuncSetAttribute(bgw_reset_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, off)) != cudaSuccess ||
         (ce = cudaFuncSetAttribute(bgw_observe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, off)) != cudaSuccess)
@@ -577,6 +580,7 @@ int bgw_specialize(bgw_handle h, const char *cache_dir)
 {
     if (!h) return fail(1, "bgw_specialize: null handle");
     if (h->jit.function || h->fast_jit.function) return 0;
+    if (h->ds.program == BGW_PROG_USER) return 0;             /* bgw_set_program compiles the program's kernel for the spec */
     /* nothing to gain (or not applicable): one of the shipped compile-time shapes; caller-supplied layouts (the compile-time
      * shapes have no layout path in their reset); the debug phase clocks (sized for the stock grid) */
     if (h->fs.enabled && (h->fast_shape != 0 || (h->bound && h->st.layout) || h->fs.prof)) return 0;
@@ -603,6 +607,20 @@ int bgw_specialize(bgw_handle h, const char *cache_dir)
     if (const char *t = getenv("BGW_GRID")) { const int v = atoi(t); if (v >= 1) h->fs.grid_ctas = std::min(h->ds.E, v); }
     h->fast_jit_on = true;
     if (getenv("BGW_VERBOSE")) fprintf(stderr, "[bgw] fast kernel compiled for this spec's shape: %d CTAs/SM, grid=%d\n", per_sm, h->fs.grid_ctas);
+    return 0;
+}
+
+int bgw_set_program(bgw_handle h, const char *source, const char *cache_dir)
+{
+    if (!h || !source) return fail(1, "bgw_set_program: null argument");
+    if (h->ds.program != BGW_PROG_USER) return fail(1, "bgw_set_program: the handle's spec runs built-in program %d, not BGW_PROG_USER", h->ds.program);
+    if (h->jit.function) return fail(1, "bgw_set_program: the handle has a step program already");
+    DeviceGuard guard(h->device);
+    CUDA_OK(cudaFree(nullptr));                              /* the runtime's primary context is current for the driver calls */
+    if (!cache_dir) cache_dir = getenv("BGW_JIT_CACHE");
+    std::string msg;
+    if (const char *e = bgwjit::build(h->ds, h->ds.init_ammo != nullptr, h->threads, cache_dir, h->jit, msg, source))
+        return fail(2, "bgw_set_program: %s", e);
     return 0;
 }
 
@@ -680,6 +698,8 @@ static void dump_prof(bgw_handle h, void *stream)
 static int step_impl(bgw_handle h, const int8_t *actions, int8_t *sampled, const int16_t *order, int8_t *obs, float *reward,
                      uint8_t *done, uint8_t *all_done, void *stream, bool chained = false, int n_steps = 1)
 {
+    if (h->ds.program == BGW_PROG_USER && !h->jit.function)
+        return fail(1, "bgw_step: the handle runs a user step program and none is installed yet (bgw_set_program)");
     DeviceGuard guard(h->device);
     if (h->randomize_action_input && !order) {
         /* all_step_manager.py:62-65: the actions are processed in shuffled order -- the keyed order of this step, written

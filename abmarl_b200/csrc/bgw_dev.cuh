@@ -488,11 +488,10 @@ static __device__ int subset_attackables_dev(const DevSpec &s, const Env &ev, co
 }
 
 /* <attack actor>._determine_attack (actor.py:455-501 Binary, 521-582 EncodingBased, 601-658 RestrictedSelective,
- * 681-728 Selective) + AttackActorBaseComponent.process_action (:306-361, with the ammo filter :343-351) + the
- * reward lines of TeamBattleSim.step (team_battle_example.py:38-47) for ONE attacker that requested an attack. */
-static __device__ void exec_attack_ext(const DevSpec &s, Env &ev, int a)
+ * 681-728 Selective) + the ammo filter of AttackActorBaseComponent.process_action (:343-351) for ONE attacker that
+ * requested an attack: victims[0..n) = attacked_agents.  Returns n. */
+static __device__ __forceinline__ int attack_victims(const DevSpec &s, Env &ev, int a, uint16_t *victims)
 {
-    if (!(ev.flags[a] & BGW_ST_ACTIVE)) return;                   /* team_battle_example.py:37 */
     AttackView v;
     v.a = a; v.R = __ldg(&s.attack_r[a]); v.n = 2 * v.R + 1;
     v.r0 = ev.cell[a] / s.W; v.c0 = ev.cell[a] % s.W;
@@ -506,7 +505,6 @@ static __device__ void exec_attack_ext(const DevSpec &s, Env &ev, int a)
     }
     const uint8_t *att = attack_bytes(s, ev, a);
     const int n = v.n, last = n - 1;
-    uint16_t victims[BGW_MAX_VICTIMS];
     int nv = 0;
     switch (s.attack_actor) {
     case BGW_ATTACK_BINARY:
@@ -557,14 +555,29 @@ static __device__ void exec_attack_ext(const DevSpec &s, Env &ev, int a)
         }
         ev.ammo[a] = max(ammo - nv, 0);
     }
-    if (nv == 0) { ev.racc[a] += s.reward[BGW_RW_ATTACK_FAIL]; return; }   /* team_battle_example.py:41-42 */
+    return nv;
+}
+
+/* the damage of process_action (actor.py:353-358): the attacked agents lose the attacker's strength, the dead leave the grid */
+static __device__ __forceinline__ void attack_damage(const DevSpec &s, Env &ev, int a, const uint16_t *victims, int nv)
+{
     const double strength = __ldg(&s.strength[a]);
-    for (int t = 0; t < nv; ++t) {                                  /* actor.py:353-358 */
+    for (int t = 0; t < nv; ++t) {
         const int x = victims[t];
         if (!(ev.flags[x] & BGW_ST_ACTIVE)) continue;
         set_health(ev, x, __ldcg(&ev.health[x]) - strength);
         if (!(ev.flags[x] & BGW_ST_ACTIVE)) { grid_unlink(ev, x); atomicAdd(&ev.ctr[CTR_KILLS], 1); }
     }
+}
+
+/* one attacker's process_action + the reward lines of TeamBattleSim.step (team_battle_example.py:37-47) */
+static __device__ void exec_attack_ext(const DevSpec &s, Env &ev, int a)
+{
+    if (!(ev.flags[a] & BGW_ST_ACTIVE)) return;                   /* team_battle_example.py:37 */
+    uint16_t victims[BGW_MAX_VICTIMS];
+    const int nv = attack_victims(s, ev, a, victims);
+    if (nv == 0) { ev.racc[a] += s.reward[BGW_RW_ATTACK_FAIL]; return; }   /* team_battle_example.py:41-42 */
+    attack_damage(s, ev, a, victims, nv);
     for (int t = 0; t < nv; ++t)                                    /* team_battle_example.py:44-47 */
         if (!(ev.flags[victims[t]] & BGW_ST_ACTIVE)) { ev.racc[victims[t]] += s.reward[BGW_RW_DIE]; ev.racc[a] += s.reward[BGW_RW_KILL]; }
 }
@@ -637,6 +650,15 @@ static __device__ bool pacman_simple_overlaps(const DevSpec &s, Env &ev, int p, 
 /* sim programs: the user-written step()                                                             */
 /* ------------------------------------------------------------------------------------------------- */
 __device__ __forceinline__ bool prog_done(const DevSpec &s, const Env &ev, int a);
+
+#ifdef BGW_USER_PROGRAM
+/* a user step program (include/bgw_program.h), compiled in at run time by bgw_set_program: defined after the program's
+ * source (bgw_program.cuh).  The hooks return -1 when the program does not define them. */
+static __device__ void user_step(const DevSpec &s, Env &ev, int nrank);
+static __device__ int user_done(const DevSpec &s, const Env &ev, int a);
+static __device__ int user_all_done(const DevSpec &s, const Env &ev);
+static __device__ double user_reward(const DevSpec &s, const Env &ev, int a, double acc);
+#endif
 
 /* ReachTheTargetSim.step reach_the_target.py:141-144: a runner standing on the target's cell has reached it.  A runner
  * that is no longer in the grid (killed on that cell) would make the reference's grid.remove raise; it is left alone. */
@@ -886,6 +908,13 @@ static __device__ void serial_program_step(const DevSpec &s, Env &ev, int nrank)
 /* get_all_done of the sim -> ctr[CTR_ALLDONE]; all threads, ends synchronised */
 static __device__ void compute_all_done(const DevSpec &s, Env &ev, int tid, int T)
 {
+#ifdef BGW_USER_PROGRAM
+    if (s.program == BGW_PROG_USER) {                               /* the program's get_all_done, else the rule below */
+        if (tid == 0) ev.ctr[CTR_ALLDONE] = user_all_done(s, ev);
+        __syncthreads();
+        if (ev.ctr[CTR_ALLDONE] >= 0) return;
+    }
+#endif
     if (s.program == BGW_PROG_MAZE) {                                /* maze_navigation.py:41-42 */
         if (tid == 0) ev.ctr[CTR_ALLDONE] = same_position(ev, s.a_nav, s.a_target);
     } else if (s.program == BGW_PROG_PACMAN || s.program == BGW_PROG_PACMAN_SIMPLE) {   /* pacman.py:140-151 */
@@ -940,6 +969,9 @@ static __device__ void compute_all_done(const DevSpec &s, Env &ev, int tid, int 
 /* get_done(agent): smart.py:106-111 / the programs' overrides */
 __device__ __forceinline__ bool prog_done(const DevSpec &s, const Env &ev, int a)
 {
+#ifdef BGW_USER_PROGRAM
+    if (s.program == BGW_PROG_USER) { const int u = user_done(s, ev, a); if (u >= 0) return u != 0; }
+#endif
     switch (s.program) {
     case BGW_PROG_MAZE: case BGW_PROG_PACMAN: case BGW_PROG_PACMAN_SIMPLE: return ev.ctr[CTR_ALLDONE] != 0;   /* maze:38-39, pacman:137-138 */
     case BGW_PROG_MULTI_MAZE: return same_position(ev, a, s.a_target);              /* multi_maze:61-64 */
@@ -1467,6 +1499,9 @@ __device__ __forceinline__ void bgw_step_body(const DevSpec &s_in, const BgwStat
     __syncthreads();
 
     /* ---- sim.step(action_dict) ------------------------------------------------------------------ */
+#ifdef BGW_USER_PROGRAM
+    if (s.program == BGW_PROG_USER) { if (tid == 0) user_step(s, ev, nrank); __syncthreads(); } else
+#endif
     if (s.program == BGW_PROG_TEAM_BATTLE || s.program == BGW_PROG_REACH_TARGET || s.program == BGW_PROG_TRAFFIC) team_battle_step(s, ev, nrank, tid, T);
     else { if (tid == 0) serial_program_step(s, ev, nrank); __syncthreads(); }
 
@@ -1482,6 +1517,9 @@ __device__ __forceinline__ void bgw_step_body(const DevSpec &s_in, const BgwStat
                 const bool dd = prog_done(s, ev, a);
                 double rr = ev.racc[a];
                 if (s.program == BGW_PROG_MULTI_MAZE && dd) rr = s.reward[BGW_RW_TARGET];   /* multi_maze:56-59 */
+#ifdef BGW_USER_PROGRAM
+                if (s.program == BGW_PROG_USER) rr = user_reward(s, ev, a, rr);
+#endif
                 ev.racc[a] = 0.0;
                 r = (float)rr;
                 d = (uint8_t)(BGW_OUT_VALID | (dd ? BGW_OUT_DONE : 0));
@@ -1539,6 +1577,9 @@ __device__ __forceinline__ void bgw_step_body(const DevSpec &s_in, const BgwStat
             const bool dd = prog_done(s, ev, a);
             double rr = ev.racc[a];
             if (s.program == BGW_PROG_MULTI_MAZE && dd) rr = s.reward[BGW_RW_TARGET];
+#ifdef BGW_USER_PROGRAM
+            if (s.program == BGW_PROG_USER) rr = user_reward(s, ev, a, rr);
+#endif
             ev.racc[a] = 0.0;
             rew[l] = (float)rr;
             dn[l] = (uint8_t)(BGW_OUT_VALID | (dd ? BGW_OUT_DONE : 0));
@@ -1553,6 +1594,9 @@ __device__ __forceinline__ void bgw_step_body(const DevSpec &s_in, const BgwStat
         uint8_t ef = 0;
         if (ev.ctr[CTR_ENVDONE]) ef |= BGW_ENV_ALL_DONE;
         if (s.horizon > 0 && (int)ev.step >= s.horizon) ef |= BGW_ENV_ALL_DONE | BGW_ENV_TRUNCATED;
+#ifdef BGW_USER_PROGRAM
+        if (ev.ctr[CTR_ERR]) { ef |= BGW_ENV_ERROR | BGW_ENV_ALL_DONE; st.error[e] = (uint32_t)ev.ctr[CTR_ERR]; }   /* bad input from the program */
+#endif
         st.step[e] = ev.step;
         st.env_flags[e] = ef;
         all_done[e] = ef;

@@ -13,7 +13,8 @@
  *     extern "C" __global__ void bgw_step_jit(...) { bgw_step_body<PROG, ATT>(...); }
  *
  * for sm_100a into a cubin, which is loaded through the driver API (libcuda.so.1, dlopen) into the primary context the
- * runtime API uses, and launched with cuLaunchKernel.  Host code only; included by bgw.cu.
+ * runtime API uses, and launched with cuLaunchKernel.  bgw_set_program compiles the same kernel with a user step program
+ * in it (bgw_program.cuh).  Host code only; included by bgw.cu.
  */
 #ifndef BGW_JIT_H_
 #define BGW_JIT_H_
@@ -167,13 +168,14 @@ inline const char *compile_and_load(std::string src, const char *name, int smem,
 {
     if (const char *e = load_driver(driver())) return e;
     const std::string dir = library_dir(), inc = dir + "/../../include";
-    std::string dev, fst, hdr, phl, sti;
-    if (!read_file(dir + "/bgw_dev.cuh", dev) || !read_file(dir + "/bgw_fast.cuh", fst) || !read_file(inc + "/bgw.h", hdr) ||
-        !read_file(inc + "/bgw_philox.h", phl) || !read_file(inc + "/bgw_stdint.h", sti)) {
-        msg = "the kernel sources (bgw_dev.cuh, bgw_fast.cuh, include/bgw*.h) are not next to the library in " + dir;
+    std::string dev, fst, prg, hdr, phl, sti, pgh;
+    if (!read_file(dir + "/bgw_dev.cuh", dev) || !read_file(dir + "/bgw_fast.cuh", fst) || !read_file(dir + "/bgw_program.cuh", prg) ||
+        !read_file(inc + "/bgw.h", hdr) || !read_file(inc + "/bgw_philox.h", phl) || !read_file(inc + "/bgw_stdint.h", sti) ||
+        !read_file(inc + "/bgw_program.h", pgh)) {
+        msg = "the kernel sources (bgw_dev.cuh, bgw_fast.cuh, bgw_program.cuh, include/bgw*.h) are not next to the library in " + dir;
         return msg.c_str();
     }
-    const unsigned long long key = fnv1a(sti, fnv1a(phl, fnv1a(hdr, fnv1a(fst, fnv1a(dev, fnv1a(src))))));
+    const unsigned long long key = fnv1a(pgh, fnv1a(sti, fnv1a(phl, fnv1a(hdr, fnv1a(prg, fnv1a(fst, fnv1a(dev, fnv1a(src))))))));
     std::string cubin, cache_path;
     if (cache_dir && *cache_dir) {
         char nm[64];
@@ -241,12 +243,17 @@ inline const char *compile_and_load(std::string src, const char *name, int smem,
     return nullptr;
 }
 
-/* the general step kernel for one spec */
-inline const char *build(const DevSpec &d, bool has_init_ammo, int threads, const char *cache_dir, Kernel &out, std::string &msg)
+/* the general step kernel for one spec; with `program` (a user step program, include/bgw_program.h) compiled into it */
+inline const char *build(const DevSpec &d, bool has_init_ammo, int threads, const char *cache_dir, Kernel &out, std::string &msg,
+                         const char *program = nullptr)
 {
     char head[1024];
     snprintf(head, sizeof(head), "#define BGW_JIT_T %d\n#define BGW_JIT_PIN ", threads);
-    std::string src = head + pin_statements(d, has_init_ammo) + "\n#include \"bgw_dev.cuh\"\n";
+    std::string src = std::string(program ? "#define BGW_USER_PROGRAM\n" : "") + head + pin_statements(d, has_init_ammo) +
+                      "\n#include \"bgw_dev.cuh\"\n";
+    if (program)   /* the program's diagnostics name its own lines */
+        src += std::string("#include \"bgw_program.cuh\"\n#line 1 \"program\"\n") + program +
+               "\n#define BGWP_AFTER_PROGRAM\n#include \"bgw_program.cuh\"\n";
     snprintf(head, sizeof(head),
              "extern \"C\" __global__ void __launch_bounds__(%d) bgw_step_jit(const DevSpec s_in, const BgwState st, const uint32_t *actions, "
              "const int16_t *order, int8_t *obs, float *reward, uint8_t *done, uint8_t *all_done)\n"

@@ -43,6 +43,9 @@ class BatchedGridWorld:
         h = C.c_void_p()
         K.check(self.lib.bgw_create(C.byref(self._c), self.device.index, C.byref(h)), self.lib)
         self._h = h
+        source = getattr(spec, 'program_source', None)
+        if source is not None:                     # the sim's own step program, compiled into the step kernel (cached in $BGW_JIT_CACHE)
+            K.check(self.lib.bgw_set_program(h, source.encode(), None), self.lib)
         d = K.BgwDims()
         K.check(self.lib.bgw_dims(h, C.byref(d)), self.lib)
         self.dims = d

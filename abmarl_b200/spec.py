@@ -12,6 +12,7 @@ import math
 import numpy as np
 
 from abmarl_b200 import _capi as K
+from abmarl_b200.program import DeviceProgram
 
 
 def _mro_names(obj):
@@ -48,6 +49,7 @@ class CompiledSpec:
         self.reward = np.zeros(K.BGW_RW_COUNT, dtype=np.float64)
         self.agent_ids = []
         self.layout_generator = None     # e.g. ('maze', params) -> host-side layouts (abmarl_b200.layouts)
+        self.program_source = None       # PROG_USER: the step program's C source (abmarl_b200.program, bgw_set_program)
 
     # ---- derived -----------------------------------------------------------------------------
     @property
@@ -133,7 +135,17 @@ def compile_sim(sim, manager='all_step', n_envs=1, env_offset=0, seed=0, horizon
     if manager == 'all_step_shuffled':                  # scenario shorthand: AllStepManager(randomize_action_input=True)
         manager, randomize_action_input = 'all_step', True
     names = _mro_names(sim)
-    sp.program = _first(names, _PROGRAMS, 'simulation class')
+    # a sim that declares its own step program runs it, whatever class it derives from (abmarl_b200.program)
+    device_program = getattr(sim, 'device_program', None)
+    program = device_program() if callable(device_program) else None
+    if program is not None:
+        if not isinstance(program, DeviceProgram):
+            raise TypeError(f"{type(sim).__name__}.device_program() must return an abmarl_b200.program.DeviceProgram")
+        if manager == 'dynamic_order':
+            raise ValueError("a device program cannot run under the DynamicOrderManager: its next_agent rule is not programmable")
+        sp.program = K.PROG_USER
+    else:
+        sp.program = _first(names, _PROGRAMS, 'simulation class')
     sp.manager = {'all_step': K.MANAGER_ALL_STEP, 'turn_based': K.MANAGER_TURN_BASED,
                   'dynamic_order': K.MANAGER_DYNAMIC_ORDER}[manager]
     if sp.manager == K.MANAGER_DYNAMIC_ORDER:
@@ -261,7 +273,10 @@ def compile_sim(sim, manager='all_step', n_envs=1, env_offset=0, seed=0, horizon
 
     # ---- program-specific roles and reward constants ----------------------------------------------
     rc = getattr(sim, 'reward_constants', {})
-    if sp.program == K.PROG_TEAM_BATTLE:        # team_battle_example.py:42-59
+    if sp.program == K.PROG_USER:               # the program carries its own constants and roles
+        sp.program_source = program.assemble(sim.agents)
+        sp.role[:] = program.role_table(sim.agents)
+    elif sp.program == K.PROG_TEAM_BATTLE:      # team_battle_example.py:42-59
         sp.reward[K.RW_ATTACK_FAIL] = rc.get('attack_fail', -0.1)
         sp.reward[K.RW_KILL] = rc.get('kill', 1.0)
         sp.reward[K.RW_DIE] = rc.get('die', -1.0)

@@ -77,7 +77,8 @@ enum {
     BGW_PROG_PACMAN = 3,      /* abmarl/examples/sim/pacman.py:29-151             */
     BGW_PROG_REACH_TARGET = 4,/* abmarl/examples/sim/reach_the_target.py:90-176   */
     BGW_PROG_TRAFFIC = 5,     /* abmarl/examples/sim/traffic_corridor.py:24-53    */
-    BGW_PROG_PACMAN_SIMPLE = 6 /* abmarl/examples/sim/pacman.py:172-326 (scripted baddies, examples/rllib_pacman.py) */
+    BGW_PROG_PACMAN_SIMPLE = 6, /* abmarl/examples/sim/pacman.py:172-326 (scripted baddies, examples/rllib_pacman.py) */
+    BGW_PROG_USER = 7          /* a user-written step program (include/bgw_program.h), installed with bgw_set_program */
 };
 
 enum { BGW_MOVE_NONE = 0, BGW_MOVE_BOX = 1 /* MoveActor actor.py:55 */, BGW_MOVE_CROSS = 2 /* :117 */,
@@ -376,6 +377,19 @@ uint64_t bgw_launch_count(bgw_handle h);
  * Results are bit-identical to the stock kernel's: it is the same source.
  */
 int bgw_specialize(bgw_handle h, const char *cache_dir);
+
+/*
+ * Install the step program of a BGW_PROG_USER handle: `source` is the program's C text (include/bgw_program.h), compiled at
+ * run time (NVRTC, sm_100a) into the general step kernel, which then runs it for every step.  Needs what bgw_specialize
+ * needs; the cubin is cached in `cache_dir` (NULL: $BGW_JIT_CACHE, else no cache) by the hash of the spec, the program and
+ * the kernel sources.  On a compile error the NVRTC diagnostic is in bgw_last_error().  Fails on a handle of any other
+ * program and when the handle has a program already.  Until a program is set, bgw_reset, bgw_observe, bgw_sample_actions
+ * and bgw_gather_valid work (they do not depend on the program) and bgw_step / bgw_step_sampled / bgw_rollout_sampled fail
+ * without touching any buffer.  A program handle never runs the specialised team-battle kernel, and bgw_specialize on it
+ * does nothing (the program's kernel is compiled for the spec already).  BGW_MANAGER_DYNAMIC_ORDER is not available to
+ * programs (its next_agent rule is not programmable).
+ */
+int bgw_set_program(bgw_handle h, const char *source, const char *cache_dir);
 
 const char *bgw_last_error(void);
 int bgw_abi_version(void);

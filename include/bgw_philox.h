@@ -53,7 +53,8 @@ enum {
      * the order the list had, and whose restriction to a sub-list is the keyed order of the sub-list */
     BGW_SITE_ORDER = 10,       /* AllStepManager(randomize_action_input) managers/all_step_manager.py:62-65 slot=agent k=0,
                                   step = the manager step that is being taken */
-    BGW_SITE_PLACE_ORDER = 11  /* PositionState(randomize_placement_order)      state.py:97-101 slot=agent k=0, step 0 */
+    BGW_SITE_PLACE_ORDER = 11, /* PositionState(randomize_placement_order)      state.py:97-101 slot=agent k=0, step 0 */
+    BGW_SITE_PROGRAM = 12      /* bgwp_uniform of a user step program (bgw_program.h)   slot, k: the program's choice */
 };
 
 BGW_HD void bgw_philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
