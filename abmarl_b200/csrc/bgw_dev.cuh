@@ -651,15 +651,6 @@ static __device__ bool pacman_simple_overlaps(const DevSpec &s, Env &ev, int p, 
 /* ------------------------------------------------------------------------------------------------- */
 __device__ __forceinline__ bool prog_done(const DevSpec &s, const Env &ev, int a);
 
-#ifdef BGW_USER_PROGRAM
-/* a user step program (include/bgw_program.h), compiled in at run time by bgw_set_program: defined after the program's
- * source (bgw_program.cuh).  The hooks return -1 when the program does not define them. */
-static __device__ void user_step(const DevSpec &s, Env &ev, int nrank);
-static __device__ int user_done(const DevSpec &s, const Env &ev, int a);
-static __device__ int user_all_done(const DevSpec &s, const Env &ev);
-static __device__ double user_reward(const DevSpec &s, const Env &ev, int a, double acc);
-#endif
-
 /* ReachTheTargetSim.step reach_the_target.py:141-144: a runner standing on the target's cell has reached it.  A runner
  * that is no longer in the grid (killed on that cell) would make the reference's grid.remove raise; it is left alone. */
 __device__ __forceinline__ void reach_check(const DevSpec &s, Env &ev, int a)
@@ -903,8 +894,28 @@ static __device__ void serial_program_step(const DevSpec &s, Env &ev, int nrank)
 }
 
 /* ------------------------------------------------------------------------------------------------- */
-/* Done components (done.py) and the programs' get_done / get_all_done                               */
+/* The sim's step / get_all_done / get_done / get_reward: built-in programs, done components         */
+/* (done.py), or a user step program                                                                 */
 /* ------------------------------------------------------------------------------------------------- */
+#ifdef BGW_USER_PROGRAM
+/* a user step program (include/bgw_program.h), compiled in at run time by bgw_set_program: defined after the program's
+ * source (bgw_program.cuh).  The hooks return -1 when the program does not define them. */
+static __device__ void user_step(const DevSpec &s, Env &ev, int nrank);
+static __device__ int user_done(const DevSpec &s, const Env &ev, int a);
+static __device__ int user_all_done(const DevSpec &s, const Env &ev);
+static __device__ double user_reward(const DevSpec &s, const Env &ev, int a, double acc);
+#endif
+
+/* sim.step(action_dict); ranks 0..nrank-1 hold the acting agents (ragent).  All threads, ends synchronised */
+__device__ __forceinline__ void prog_step(const DevSpec &s, Env &ev, int nrank, int tid, int T)
+{
+#ifdef BGW_USER_PROGRAM
+    if (s.program == BGW_PROG_USER) { if (tid == 0) user_step(s, ev, nrank); __syncthreads(); return; }
+#endif
+    if (s.program == BGW_PROG_TEAM_BATTLE || s.program == BGW_PROG_REACH_TARGET || s.program == BGW_PROG_TRAFFIC) team_battle_step(s, ev, nrank, tid, T);
+    else { if (tid == 0) serial_program_step(s, ev, nrank); __syncthreads(); }
+}
+
 /* get_all_done of the sim -> ctr[CTR_ALLDONE]; all threads, ends synchronised */
 static __device__ void compute_all_done(const DevSpec &s, Env &ev, int tid, int T)
 {
@@ -987,6 +998,19 @@ __device__ __forceinline__ bool prog_done(const DevSpec &s, const Env &ev, int a
         return d;
     }
     }
+}
+
+/* get_reward(agent) of an agent whose get_done is dd: read-and-zero smart.py:101-104, the MultiMaze override
+ * multi_maze_navigation.py:56-59, the program's hook */
+__device__ __forceinline__ double prog_take_reward(const DevSpec &s, Env &ev, int a, bool dd)
+{
+    double r = ev.racc[a];
+    if (s.program == BGW_PROG_MULTI_MAZE && dd) r = s.reward[BGW_RW_TARGET];
+#ifdef BGW_USER_PROGRAM
+    if (s.program == BGW_PROG_USER) r = user_reward(s, ev, a, r);
+#endif
+    ev.racc[a] = 0.0;
+    return r;
 }
 
 /* ------------------------------------------------------------------------------------------------- */
@@ -1498,13 +1522,7 @@ __device__ __forceinline__ void bgw_step_body(const DevSpec &s_in, const BgwStat
     }
     __syncthreads();
 
-    /* ---- sim.step(action_dict) ------------------------------------------------------------------ */
-#ifdef BGW_USER_PROGRAM
-    if (s.program == BGW_PROG_USER) { if (tid == 0) user_step(s, ev, nrank); __syncthreads(); } else
-#endif
-    if (s.program == BGW_PROG_TEAM_BATTLE || s.program == BGW_PROG_REACH_TARGET || s.program == BGW_PROG_TRAFFIC) team_battle_step(s, ev, nrank, tid, T);
-    else { if (tid == 0) serial_program_step(s, ev, nrank); __syncthreads(); }
-
+    prog_step(s, ev, nrank, tid, T);                                /* sim.step(action_dict) */
     compute_all_done(s, ev, tid, T);
 
     /* ---- who receives (obs, reward, done) -------------------------------------------------------- */
@@ -1515,13 +1533,7 @@ __device__ __forceinline__ void bgw_step_body(const DevSpec &s_in, const BgwStat
             if (!(ev.flags[a] & BGW_ST_DONE_REPORTED)) {
                 ev.plist[atomicAdd(&ev.ctr[CTR_NEMIT], 1)] = (uint16_t)l;
                 const bool dd = prog_done(s, ev, a);
-                double rr = ev.racc[a];
-                if (s.program == BGW_PROG_MULTI_MAZE && dd) rr = s.reward[BGW_RW_TARGET];   /* multi_maze:56-59 */
-#ifdef BGW_USER_PROGRAM
-                if (s.program == BGW_PROG_USER) rr = user_reward(s, ev, a, rr);
-#endif
-                ev.racc[a] = 0.0;
-                r = (float)rr;
+                r = (float)prog_take_reward(s, ev, a, dd);
                 d = (uint8_t)(BGW_OUT_VALID | (dd ? BGW_OUT_DONE : 0));
                 if (dd) ev.flags[a] |= BGW_ST_DONE_REPORTED;
                 else atomicAdd(&ev.ctr[CTR_REMAINING], 1);
@@ -1575,13 +1587,7 @@ __device__ __forceinline__ void bgw_step_body(const DevSpec &s_in, const BgwStat
         for (int i = tid; i < ev.ctr[CTR_NEMIT]; i += T) {
             const int l = ev.plist[i], a = __ldg(&s.agent_of[l]);
             const bool dd = prog_done(s, ev, a);
-            double rr = ev.racc[a];
-            if (s.program == BGW_PROG_MULTI_MAZE && dd) rr = s.reward[BGW_RW_TARGET];
-#ifdef BGW_USER_PROGRAM
-            if (s.program == BGW_PROG_USER) rr = user_reward(s, ev, a, rr);
-#endif
-            ev.racc[a] = 0.0;
-            rew[l] = (float)rr;
+            rew[l] = (float)prog_take_reward(s, ev, a, dd);
             dn[l] = (uint8_t)(BGW_OUT_VALID | (dd ? BGW_OUT_DONE : 0));
         }
         __syncthreads();

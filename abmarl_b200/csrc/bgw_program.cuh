@@ -11,10 +11,10 @@
  *     #include "bgw_program.cuh"        user_step / user_done / ... : the engine's calls into the program
  *     <kernel wrapper>
  *
- * The program runs on thread 0 of the env's CTA between two barriers (bgw_step_body), like the built-in serial programs,
+ * The program runs on thread 0 of the env's CTA between two barriers (prog_step), like the built-in serial programs,
  * so the API functions are the serial primitives of bgw_dev.cuh: process_move, try_move, grid_query, grid_append,
- * grid_unlink, set_health, dev_draw and the attack code.  The oracle (tests/program_oracle.c) implements the same API over
- * its own primitives.
+ * grid_unlink, set_health, dev_draw and the attack code.  The oracle (oracle/bgw_oracle_program.c) implements the same API
+ * over its own primitives.
  */
 #ifndef BGWP_AFTER_PROGRAM
 

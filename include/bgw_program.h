@@ -5,7 +5,7 @@
  * step(action_dict) and, sometimes, get_done / get_all_done / get_reward (abmarl/sim/agent_based_simulation.py:238-294).
  * Here that code is ONE C source text, a "step program".  It is compiled twice from the same text:
  *   - by NVRTC as CUDA C++ into the general step kernel (bgw_set_program, include/bgw.h; abmarl_b200/csrc/bgw_program.cuh),
- *   - by gcc as C into the CPU oracle (tests/program_oracle.c over oracle/bgw_oracle.c), which checks it bit for bit.
+ *   - by gcc as C into the CPU oracle (oracle/bgw_oracle_program.c over oracle/bgw_oracle.c), which checks it bit for bit.
  * So a program is written in the common subset of C99 and C++17: no references, templates, classes, `bool` or library calls.
  * Its own functions are declared with BGWP_FN.
  *

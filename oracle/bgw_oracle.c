@@ -37,6 +37,11 @@ typedef struct {
     int *agent_of;    /* [L] agent index */
     uint8_t *mask;    /* LOS scratch */
     int mask_cap;
+    /* the step in progress (bgwo_step) */
+    int *acting;      /* [n_acting] agent per acting slot in processing order, -1 = reported done already */
+    int n_acting;
+    const int8_t *actions;   /* this env's action rows */
+    uint32_t err;     /* bad input from a step program: BgwState.error at the end of the step (the step kernel's CTR_ERR) */
 } Ctx;
 
 /* ------------------------------------------------------------------------------------------------- */
@@ -549,6 +554,15 @@ static int same_position(const Ctx *c, int a, int b) { return c->cell[a] == c->c
 
 static int prog_all_done(const Ctx *c);
 
+#ifdef BGW_USER_PROGRAM
+/* a user step program (include/bgw_program.h), compiled in by build_program (oracle/build.py): defined after the program's
+ * source (bgw_oracle_program.c).  The hooks return -1 when the program does not define them. */
+static void user_step(Ctx *c);
+static int user_done(const Ctx *c, int a);
+static int user_all_done(const Ctx *c);
+static double user_reward(const Ctx *c, int a, double acc);
+#endif
+
 /* PacmanSimSimple.step pacman.py:235-303: the baddies' scripted DriftMoveActor actions for this step.  k indexes the
  * script's entries (baddie_20, 36, 156, 157, 159, 161, 162, 206, 222, 328); sc = step_count; o156 = orientation of
  * baddie_156; x159 = the keyed draw that stands in for np.random.randint(0, 5) */
@@ -619,6 +633,9 @@ static int learners_remaining(const Ctx *c)
 
 static int prog_done(const Ctx *c, int a)
 {
+#ifdef BGW_USER_PROGRAM
+    if (c->sp->program == BGW_PROG_USER) { const int u = user_done(c, a); if (u >= 0) return u; }
+#endif
     switch (c->sp->program) {
     case BGW_PROG_REACH_TARGET: {                                                   /* reach_the_target.py:161-168 */
         const int t = find_role(c, BGW_ROLE_TARGET);
@@ -636,6 +653,9 @@ static int prog_done(const Ctx *c, int a)
 
 static int prog_all_done(const Ctx *c)
 {
+#ifdef BGW_USER_PROGRAM
+    if (c->sp->program == BGW_PROG_USER) { const int u = user_all_done(c); if (u >= 0) return u; }
+#endif
     switch (c->sp->program) {
     case BGW_PROG_REACH_TARGET: return learners_remaining(c) <= 1;                  /* reach_the_target.py:170-171,56-57 */
     case BGW_PROG_MAZE:                                                             /* maze_navigation.py:41-42 */
@@ -656,11 +676,14 @@ static int prog_all_done(const Ctx *c)
     }
 }
 
-/* get_reward: read-and-zero smart.py:101-104; MultiMaze override multi_maze_navigation.py:56-59 */
+/* get_reward: read-and-zero smart.py:101-104; MultiMaze override multi_maze_navigation.py:56-59; a program's hook */
 static double prog_take_reward(Ctx *c, int a)
 {
     double r = c->racc[a];
     if (c->sp->program == BGW_PROG_MULTI_MAZE && prog_done(c, a)) r = c->sp->reward[BGW_RW_TARGET];
+#ifdef BGW_USER_PROGRAM
+    if (c->sp->program == BGW_PROG_USER) r = user_reward(c, a, r);
+#endif
     c->racc[a] = 0.0;
     return r;
 }
@@ -698,57 +721,53 @@ static void pacman_overlaps(Ctx *c, int p, int eat_food)   /* pacman.py:94-105,1
     }
 }
 
-/* `acting[i]` = agent indices that submitted an action, in action_dict order; act(i) their 4 bytes */
-static void prog_step(Ctx *c, const int *acting, int n_act, const int8_t *actions)
+#define ACT(a) (c->actions + (size_t)c->learner_of[(a)] * c->astride)
+
+/* the attack phase of TeamBattleSim.step team_battle_example.py:35-47 and ReachTheTargetSim.step reach_the_target.py:119-131 */
+static void attack_phase(Ctx *c)
+{
+    const double *rw = c->sp->reward;
+    int victims[BGW_MAX_VICTIMS + 1];
+    for (int i = 0; i < c->n_acting; ++i) {
+        const int a = c->acting[i];
+        if (a < 0 || !(c->flags[a] & BGW_ST_ACTIVE)) continue;
+        int nv = 0;
+        const int status = process_attack(c, a, (const uint8_t *)ACT(a) + 2, victims, &nv);
+        if (status) {
+            if (nv == 0) c->racc[a] += rw[BGW_RW_ATTACK_FAIL];
+            else for (int t = 0; t < nv; ++t)
+                if (!(c->flags[victims[t]] & BGW_ST_ACTIVE)) {
+                    c->racc[victims[t]] += rw[BGW_RW_DIE];
+                    c->racc[a] += rw[BGW_RW_KILL];
+                }
+        }
+    }
+}
+
+/* sim.step(action_dict) over the acting set c->acting[0 .. n_acting) (agents in action_dict order; -1: no action, the
+ * learner was reported done already) and their action rows */
+static void prog_step(Ctx *c)
 {
     const BgwSpec *sp = c->sp;
     const double *rw = sp->reward;
-#define ACT(a) (actions + (size_t)c->learner_of[(a)] * c->astride)
+    const int n_act = c->n_acting, *acting = c->acting;
     switch (sp->program) {
     case BGW_PROG_TEAM_BATTLE: {                               /* team_battle_example.py:33-59 */
-        int victims[BGW_MAX_VICTIMS + 1];
-        for (int i = 0; i < n_act; ++i) {                      /* :35-47 */
-            const int a = acting[i];
-            if (!(c->flags[a] & BGW_ST_ACTIVE)) continue;
-            int nv = 0;
-            const int status = process_attack(c, a, (const uint8_t *)ACT(a) + 2, victims, &nv);
-            if (status) {
-                if (nv == 0) c->racc[a] += rw[BGW_RW_ATTACK_FAIL];
-                else for (int t = 0; t < nv; ++t)
-                    if (!(c->flags[victims[t]] & BGW_ST_ACTIVE)) {
-                        c->racc[victims[t]] += rw[BGW_RW_DIE];
-                        c->racc[a] += rw[BGW_RW_KILL];
-                    }
-            }
-        }
+        attack_phase(c);                                       /* :35-47 */
         for (int i = 0; i < n_act; ++i) {                      /* :50-55 */
             const int a = acting[i];
-            if (!(c->flags[a] & BGW_ST_ACTIVE)) continue;
+            if (a < 0 || !(c->flags[a] & BGW_ST_ACTIVE)) continue;
             if (!process_move(c, a, ACT(a))) c->racc[a] += rw[BGW_RW_MOVE_FAIL];
         }
-        for (int i = 0; i < n_act; ++i) c->racc[acting[i]] += rw[BGW_RW_ENTROPY];   /* :58-59 */
+        for (int i = 0; i < n_act; ++i) if (acting[i] >= 0) c->racc[acting[i]] += rw[BGW_RW_ENTROPY];   /* :58-59 */
         break;
     }
     case BGW_PROG_REACH_TARGET: {                              /* reach_the_target.py:117-152 */
-        int victims[BGW_MAX_VICTIMS + 1];
         const int tgt = find_role(c, BGW_ROLE_TARGET);
-        for (int i = 0; i < n_act; ++i) {                      /* :119-131 (same shape as the team battle) */
-            const int a = acting[i];
-            if (!(c->flags[a] & BGW_ST_ACTIVE)) continue;
-            int nv = 0;
-            const int status = process_attack(c, a, (const uint8_t *)ACT(a) + 2, victims, &nv);
-            if (status) {
-                if (nv == 0) c->racc[a] += rw[BGW_RW_ATTACK_FAIL];
-                else for (int t = 0; t < nv; ++t)
-                    if (!(c->flags[victims[t]] & BGW_ST_ACTIVE)) {
-                        c->racc[victims[t]] += rw[BGW_RW_DIE];
-                        c->racc[a] += rw[BGW_RW_KILL];
-                    }
-            }
-        }
+        attack_phase(c);                                       /* :119-131 */
         for (int i = 0; i < n_act; ++i) {                      /* :134-145 */
             const int a = acting[i];
-            if (!(sp->klass[a] & BGW_AG_MOVING)) continue;
+            if (a < 0 || !(sp->klass[a] & BGW_AG_MOVING)) continue;
             if (c->flags[a] & BGW_ST_ACTIVE)
                 if (!process_move(c, a, ACT(a))) c->racc[a] += rw[BGW_RW_MOVE_FAIL];
             /* TargetDone.get_done :33-40.  A runner that is no longer in the grid (killed while standing on the
@@ -760,12 +779,13 @@ static void prog_step(Ctx *c, const int *acting, int n_act, const int8_t *action
             }
         }
         for (int i = 0; i < n_act; ++i)                         /* :148-150 */
-            if (sp->role[acting[i]] == BGW_ROLE_RUNNER) c->racc[acting[i]] += rw[BGW_RW_ENTROPY];
+            if (acting[i] >= 0 && sp->role[acting[i]] == BGW_ROLE_RUNNER) c->racc[acting[i]] += rw[BGW_RW_ENTROPY];
         break;
     }
     case BGW_PROG_TRAFFIC:                                     /* traffic_corridor.py:46-53 */
         for (int i = 0; i < n_act; ++i) {
             const int a = acting[i];
+            if (a < 0) continue;
             if (!process_move(c, a, ACT(a))) c->racc[a] += rw[BGW_RW_MOVE_FAIL];
             if (smart_done(c, a)) c->racc[a] += rw[BGW_RW_TARGET];
         }
@@ -780,6 +800,7 @@ static void prog_step(Ctx *c, const int *acting, int n_act, const int8_t *action
     case BGW_PROG_MULTI_MAZE: {                                /* multi_maze_navigation.py:40-48 */
         for (int i = 0; i < n_act; ++i) {
             const int a = acting[i];
+            if (a < 0) continue;
             if (!process_move(c, a, ACT(a))) c->racc[a] += rw[BGW_RW_MOVE_FAIL];
             c->racc[a] += rw[BGW_RW_ENTROPY];
         }
@@ -836,7 +857,7 @@ static void prog_step(Ctx *c, const int *acting, int n_act, const int8_t *action
         pacman_overlaps(c, p, 1);
         for (int i = 0; i < n_act; ++i) {
             const int a = acting[i];
-            if (a == p) continue;
+            if (a < 0 || a == p) continue;
             if (!process_move(c, a, ACT(a))) c->racc[a] += rw[BGW_RW_MOVE_FAIL];
             else c->racc[a] += rw[BGW_RW_ENTROPY];
             pacman_teleport(c, a);
@@ -845,10 +866,13 @@ static void prog_step(Ctx *c, const int *acting, int n_act, const int8_t *action
         if (!(c->flags[p] & BGW_ST_ACTIVE)) grid_remove(c, p);  /* :134-135 */
         break;
     }
+#ifdef BGW_USER_PROGRAM
+    case BGW_PROG_USER: user_step(c); break;
+#endif
     default: break;
     }
-#undef ACT
 }
+#undef ACT
 
 /* ------------------------------------------------------------------------------------------------- */
 /* State components: state.py                                                                        */
@@ -1029,20 +1053,30 @@ static void emit(Ctx *c, int l, int8_t *obs_env, int stride, float *rew, double 
     c->st->stats[(size_t)c->env * BGW_STAT_COUNT + BGW_STAT_AGENT_STEPS]++;
 }
 
+/* One manager step of every env.  A step program (BGW_PROG_USER) needs the library built with it (build_program) and runs
+ * under the all-step and turn-based managers; otherwise nothing is touched and the result is non-zero.  Bad input from
+ * the program ends the env with BgwState.error = 3 (bgw_program.h). */
 int bgwo_step(const BgwSpec *sp, BgwState *st, const int8_t *actions, const int16_t *order, int8_t *obs,
               float *reward, double *reward64, uint8_t *done, uint8_t *all_done)
 {
+    if (sp->program == BGW_PROG_USER) {
+#ifndef BGW_USER_PROGRAM
+        return 1;
+#endif
+        if (sp->manager == BGW_MANAGER_DYNAMIC_ORDER) return 1;
+    }
     Ctx c; ctx_init(&c, sp, st);
     BgwDims d; bgwo_dims(sp, &d);
     const int L = c.L, stride = d.obs_stride;
-    int *acting = (int *)malloc(sizeof(int) * (size_t)(L + 1));
+    c.acting = (int *)malloc(sizeof(int) * (size_t)(L + 1));
     for (int e = 0; e < sp->n_envs; ++e) {
         ctx_env(&c, e);
         int8_t *obs_env = obs ? obs + (size_t)e * L * stride : NULL;
         float *rew = reward ? reward + (size_t)e * L : NULL;
         double *rew64 = reward64 ? reward64 + (size_t)e * L : NULL;
         uint8_t *dn = done + (size_t)e * L;
-        const int8_t *act = actions + (size_t)e * L * c.astride;
+        c.actions = actions + (size_t)e * L * c.astride;
+        c.err = 0;
         for (int l = 0; l < L; ++l) { dn[l] = 0; if (rew) rew[l] = 0.f; if (rew64) rew64[l] = 0.0; }
 
         if (st->env_flags[e] & BGW_ENV_ALL_DONE) {
@@ -1059,15 +1093,14 @@ int bgwo_step(const BgwSpec *sp, BgwState *st, const int8_t *actions, const int1
         int env_done = 0;
 
         if (sp->manager == BGW_MANAGER_ALL_STEP) {              /* all_step_manager.py:51-95 */
-            int n_act = 0;
-            for (int i = 0; i < L; ++i) {
-                const int l = order ? order[(size_t)e * L + i] : i;
-                const int a = c.agent_of[l];
-                if (!(c.flags[a] & BGW_ST_DONE_REPORTED)) acting[n_act++] = a;
-            }
-            /* all_step_manager.py:62-65: the submitted actions in shuffled order (the keyed order of this step) */
-            if (!order && sp->randomize_action_input) keyed_order(&c, BGW_SITE_ORDER, st->step[e], acting, n_act);
-            prog_step(&c, acting, n_act, act);                  /* :66 */
+            /* one acting slot per learner in processing order: dict order, the caller's, or (:62-65) the keyed order of
+             * this step.  A learner reported done sends no action (:59-61): its slot holds -1.  The keyed order of the
+             * others is the restriction of the full one, so it is taken before they are marked. */
+            for (int i = 0; i < L; ++i) c.acting[i] = c.agent_of[order ? order[(size_t)e * L + i] : i];
+            if (!order && sp->randomize_action_input) keyed_order(&c, BGW_SITE_ORDER, st->step[e], c.acting, L);
+            for (int i = 0; i < L; ++i) if (c.flags[c.acting[i]] & BGW_ST_DONE_REPORTED) c.acting[i] = -1;
+            c.n_acting = L;
+            prog_step(&c);                                      /* :66 */
             for (int l = 0; l < L; ++l) {                       /* :68-87 */
                 const int a = c.agent_of[l];
                 if (c.flags[a] & BGW_ST_DONE_REPORTED) continue;
@@ -1082,8 +1115,9 @@ int bgwo_step(const BgwSpec *sp, BgwState *st, const int8_t *actions, const int1
             env_done = prog_all_done(&c) || remaining == 0;     /* :90-93 */
         } else {                                                /* turn_based_manager.py:34-94 */
             int l = st->turn[e];
-            acting[0] = c.agent_of[l];
-            prog_step(&c, acting, 1, act);                      /* :46 */
+            c.acting[0] = c.agent_of[l];
+            c.n_acting = 1;
+            prog_step(&c);                                      /* :46 */
             env_done = prog_all_done(&c);                       /* :48 */
             if (env_done) {                                     /* :49-57, dynamic_order_manager.py:43-51 */
                 for (int k = 0; k < L; ++k)
@@ -1127,11 +1161,12 @@ int bgwo_step(const BgwSpec *sp, BgwState *st, const int8_t *actions, const int1
         uint8_t ef = 0;
         if (env_done) ef |= BGW_ENV_ALL_DONE;
         if (sp->horizon > 0 && (int)st->step[e] >= sp->horizon) ef |= BGW_ENV_ALL_DONE | BGW_ENV_TRUNCATED;
+        if (c.err) { ef |= BGW_ENV_ERROR | BGW_ENV_ALL_DONE; st->error[e] = c.err; }
         if (ef & BGW_ENV_ALL_DONE) st->stats[(size_t)e * BGW_STAT_COUNT + BGW_STAT_EPISODES]++;
         st->env_flags[e] = ef;
         all_done[e] = ef;
     }
-    free(acting);
+    free(c.acting);
     ctx_free(&c);
     return 0;
 }

@@ -1,30 +1,36 @@
 """ctypes front-end of the C oracle (oracle/bgw_oracle.c).  TEST INFRASTRUCTURE ONLY.
 
 OracleEnv mirrors abmarl_b200.engine.BatchedGridWorld on numpy arrays so the parity tests can drive both
-with the same code and compare array for array.
+with the same code and compare array for array.  A spec with a step program (CompiledSpec.program_source) runs on the
+oracle built with that program (build_program).
 """
 import ctypes as C
 
 import numpy as np
 
 from abmarl_b200 import _capi as K
-from oracle.build import build
+from oracle.build import build, build_program
 
-_LIB = None
+_LIBS = {}          # program source (None: the plain oracle) -> loaded library
 
 
-def lib():
-    global _LIB
-    if _LIB is None:
-        _LIB = C.CDLL(build())
-        p = C.c_void_p
-        _LIB.bgwo_dims.argtypes = [C.POINTER(K.BgwSpec), C.POINTER(K.BgwDims)]
-        _LIB.bgwo_reset.argtypes = [C.POINTER(K.BgwSpec), C.POINTER(K.BgwState), p, p]
-        _LIB.bgwo_step.argtypes = [C.POINTER(K.BgwSpec), C.POINTER(K.BgwState), p, p, p, p, p, p, p]
-        _LIB.bgwo_sample_actions.argtypes = [C.POINTER(K.BgwSpec), C.POINTER(K.BgwState), p]
-        _LIB.bgwo_los_mask.argtypes = [C.c_int, C.c_int, C.c_int, p]
-        _LIB.bgwo_observe.argtypes = [C.POINTER(K.BgwSpec), C.POINTER(K.BgwState), C.c_int, p]
-    return _LIB
+def _load(path):
+    lib = C.CDLL(path)
+    p = C.c_void_p
+    lib.bgwo_dims.argtypes = [C.POINTER(K.BgwSpec), C.POINTER(K.BgwDims)]
+    lib.bgwo_reset.argtypes = [C.POINTER(K.BgwSpec), C.POINTER(K.BgwState), p, p]
+    lib.bgwo_step.argtypes = [C.POINTER(K.BgwSpec), C.POINTER(K.BgwState), p, p, p, p, p, p, p]
+    lib.bgwo_sample_actions.argtypes = [C.POINTER(K.BgwSpec), C.POINTER(K.BgwState), p]
+    lib.bgwo_los_mask.argtypes = [C.c_int, C.c_int, C.c_int, p]
+    lib.bgwo_observe.argtypes = [C.POINTER(K.BgwSpec), C.POINTER(K.BgwState), C.c_int, p]
+    return lib
+
+
+def lib(program_source=None):
+    """The plain oracle, or the oracle built with a step program."""
+    if program_source not in _LIBS:
+        _LIBS[program_source] = _load(build() if program_source is None else build_program(program_source))
+    return _LIBS[program_source]
 
 
 def _ptr(a):
@@ -63,8 +69,9 @@ class OracleEnv:
     def __init__(self, spec):
         self.spec = spec
         self._c = spec.c_struct()
+        self._lib = lib(spec.program_source)
         d = K.BgwDims()
-        lib().bgwo_dims(C.byref(self._c), C.byref(d))
+        self._lib.bgwo_dims(C.byref(self._c), C.byref(d))
         self.dims = d
         self.E, self.A, self.L = spec.n_envs, spec.n_agents, d.n_learners
         self.state = alloc_state(self.E, self.A)
@@ -87,13 +94,13 @@ class OracleEnv:
     def reset(self, env_mask=None):
         m = None if env_mask is None else np.ascontiguousarray(env_mask, dtype=np.uint8)
         s = self._state_struct()
-        lib().bgwo_reset(C.byref(self._c), C.byref(s), _ptr(m), _ptr(self.obs))
+        self._lib.bgwo_reset(C.byref(self._c), C.byref(s), _ptr(m), _ptr(self.obs))
         return self.obs
 
     def sample_actions(self):
         act = np.zeros((self.E, self.L, self.dims.action_stride), dtype=np.int8)
         s = self._state_struct()
-        lib().bgwo_sample_actions(C.byref(self._c), C.byref(s), _ptr(act))
+        self._lib.bgwo_sample_actions(C.byref(self._c), C.byref(s), _ptr(act))
         return act
 
     def step(self, actions, order=None):
@@ -101,14 +108,15 @@ class OracleEnv:
         assert actions.shape == (self.E, self.L, self.dims.action_stride)
         o = None if order is None else np.ascontiguousarray(order, dtype=np.int16)
         s = self._state_struct()
-        lib().bgwo_step(C.byref(self._c), C.byref(s), _ptr(actions), _ptr(o), _ptr(self.obs), _ptr(self.reward),
-                        _ptr(self.reward64), _ptr(self.done), _ptr(self.all_done))
+        rc = self._lib.bgwo_step(C.byref(self._c), C.byref(s), _ptr(actions), _ptr(o), _ptr(self.obs), _ptr(self.reward),
+                                 _ptr(self.reward64), _ptr(self.done), _ptr(self.all_done))
+        assert rc == 0, "the oracle runs a step program under the all-step and turn-based managers only"
         return self.obs, self.reward, self.done, self.all_done
 
     def observe(self, env=0):
         out = np.zeros((self.L, self.dims.obs_stride), dtype=np.int8)
         s = self._state_struct()
-        lib().bgwo_observe(C.byref(self._c), C.byref(s), env, _ptr(out))
+        self._lib.bgwo_observe(C.byref(self._c), C.byref(s), env, _ptr(out))
         return out
 
     # ---- helpers shared with the tests ---------------------------------------------------------

@@ -13,6 +13,7 @@ from abmarl_b200 import _capi as K
 from abmarl_b200.examples.foraging import ForagingSim
 from abmarl_b200.program import DeviceProgram
 from abmarl_b200.spec import compile_sim
+from oracle.oracle import OracleEnv
 from tests import program_cases as P
 from tests.helpers import assert_outputs_equal, assert_state_equal, run_lockstep
 
@@ -32,11 +33,6 @@ def _jit_cache(tmp_path_factory):
 def _engine(spec):
     from abmarl_b200.engine import BatchedGridWorld
     return BatchedGridWorld(spec, device='cuda:0')
-
-
-def _oracle(spec):
-    from tests.program_oracle import ProgramOracleEnv
-    return ProgramOracleEnv(spec)
 
 
 # the scenario sizes of test_gpu_parity.CASES (tb_c5, the 64x64 headline shape, which that list leaves to other tests: 16 envs)
@@ -84,7 +80,7 @@ def test_program_on_the_engine(name):
     E, steps, horizon = CASES[name]
     base, spec = P.specs(name, n_envs=E, env_offset=7, seed=0xC0FFEE, horizon=horizon, auto_reset=True)
     eng = _engine(spec)
-    n = run_lockstep(eng, _oracle(spec), steps, label=f'program/{name}')
+    n = run_lockstep(eng, OracleEnv(spec), steps, label=f'program/{name}')
     assert n > 0 and int(eng.stats()[K.STAT_AGENT_STEPS].item()) == n
     # (3) against the built-in program on the engine (its own kernel: the specialised team-battle one where it qualifies)
     a, b = _engine(base), _engine(spec)
@@ -110,7 +106,7 @@ def test_program_on_the_engine(name):
 def test_foraging_engine_matches_oracle(manager, shuffled):
     spec = compile_sim(ForagingSim.build(), manager=manager, n_envs=128, env_offset=11, seed=2024, horizon=40, auto_reset=True,
                        randomize_action_input=shuffled)
-    eng, ora = _engine(spec), _oracle(spec)
+    eng, ora = _engine(spec), OracleEnv(spec)
     n = run_lockstep(eng, ora, 300, label=f'foraging/{manager}/{shuffled}')
     assert n > 0
     st = ora.state
@@ -198,7 +194,7 @@ def test_step_before_set_program_fails_and_writes_nothing():
     eng.sample_actions()
     eng.specialize()
     K.check(eng.lib.bgw_set_program(eng._h, spec.program_source.encode(), None), eng.lib)
-    ora = _oracle(spec)
+    ora = OracleEnv(spec)
     ora.reset()
     for t in range(20):
         eng.step(eng.sample_actions())

@@ -2,6 +2,7 @@
 the unmodified reference when the program re-expresses the reference's step(), runs in lockstep with the built-in program,
 runs ForagingSim (a sim no built-in program expresses) to a hand-computed answer, and guards against bad input; every
 program compiles under NVRTC for sm_100a as the engine assembles it; compile_sim / DeviceProgram checks."""
+import copy
 import ctypes as C
 import os
 import subprocess
@@ -13,8 +14,8 @@ from abmarl_b200 import _capi as K
 from abmarl_b200.examples.foraging import Forager, ForagingSim, Predator, Resource
 from abmarl_b200.program import DeviceProgram
 from abmarl_b200.spec import compile_sim
-from oracle.oracle import OracleEnv, lib as oracle_lib
-from tests.program_oracle import ProgramOracleEnv, build_program
+from oracle.build import build_program
+from oracle.oracle import OracleEnv, _ptr, lib as oracle_lib
 from tests import program_cases as P
 from tests import scenarios
 from tests.helpers import assert_state_equal
@@ -27,7 +28,7 @@ def test_program_reproduces_reference_transcript(name):
     """The checks of test_engine_reproduces_reference_transcript, on the oracle built with the re-expressed program."""
     g = np.load(os.path.join(GOLDEN, name + '.npz'))
     _, spec = P.specs(name, n_envs=1, seed=int(g['seed']), auto_reset=False)
-    ora = ProgramOracleEnv(spec)
+    ora = OracleEnv(spec)
     n_valid, episode = 0, -1
     for t in range(len(g['kind'])):
         present = g['obs_present'][t]
@@ -90,7 +91,7 @@ def _lockstep(a, b, steps, label, order_fn=None):
 def test_program_runs_in_lockstep_with_builtin_program(name):
     """16 envs, 120 steps, auto-reset: the program and the built-in program give identical state, obs, float64 rewards, dones."""
     base, prog = P.specs(name, n_envs=16, env_offset=5, seed=0xBEEF, horizon=30, auto_reset=True)
-    episodes = _lockstep(OracleEnv(base), ProgramOracleEnv(prog), 120, name)
+    episodes = _lockstep(OracleEnv(base), OracleEnv(prog), 120, name)
     assert episodes > 0
 
 
@@ -99,7 +100,7 @@ def test_program_lockstep_with_caller_order():
     base, prog = P.specs('tb_c2', n_envs=16, seed=11, horizon=40, auto_reset=True)
     rng = np.random.default_rng(0)
     orders = [np.stack([rng.permutation(base.n_learners) for _ in range(16)]).astype(np.int16) for _ in range(100)]
-    _lockstep(OracleEnv(base), ProgramOracleEnv(prog), 100, 'tb_c2/order', order_fn=lambda t: orders[t])
+    _lockstep(OracleEnv(base), OracleEnv(prog), 100, 'tb_c2/order', order_fn=lambda t: orders[t])
 
 
 # ---- ForagingSim ---------------------------------------------------------------------------------------------------------
@@ -118,7 +119,7 @@ def test_foraging_known_answer():
     sim = _foraging_kat_sim()
     spec = compile_sim(sim, n_envs=1, seed=1234)
     assert spec.program == K.PROG_USER and list(spec.role) == [1, 1, 2, 3]
-    ora = ProgramOracleEnv(spec)
+    ora = OracleEnv(spec)
     ora.reset()
     np.testing.assert_array_equal(ora.state['health'][0], [1.0, 1.0, 0.0, 0.25])
     act = np.zeros((1, 3, 4), dtype=np.int8)          # learners f0, f1, p0: [dr, dc, attack, 0]
@@ -152,7 +153,7 @@ def test_foraging_known_answer():
 
 def test_foraging_runs_200_steps_without_error():
     spec = compile_sim(ForagingSim.build(), n_envs=16, env_offset=3, seed=9, horizon=60, auto_reset=True)
-    ora = ProgramOracleEnv(spec)
+    ora = OracleEnv(spec)
     ora.reset()
     episodes = 0
     for t in range(200):
@@ -164,13 +165,32 @@ def test_foraging_runs_200_steps_without_error():
     assert ora.state['stats'][:, K.STAT_KILLS].sum() > 0
 
 
+def test_oracle_without_the_program_refuses_to_step_it():
+    """The plain oracle refuses to step a spec with a step program and writes nothing; OracleEnv(spec) runs the program."""
+    spec = compile_sim(ForagingSim.build(), n_envs=2, seed=1)
+    ora = OracleEnv(spec)
+    ora.reset()
+    act = ora.sample_actions()
+    state = copy.deepcopy(ora.state)
+    outputs = [x.copy() for x in (ora.obs, ora.reward64, ora.done, ora.all_done)]
+    rc = oracle_lib().bgwo_step(C.byref(ora._c), C.byref(ora._state_struct()), _ptr(act), None, _ptr(ora.obs), _ptr(ora.reward),
+                                _ptr(ora.reward64), _ptr(ora.done), _ptr(ora.all_done))
+    assert rc != 0
+    assert_state_equal(ora.state, state, 'refused step')
+    for x, y in zip((ora.obs, ora.reward64, ora.done, ora.all_done), outputs):
+        np.testing.assert_array_equal(x, y)
+    ora.step(act)
+    assert (ora.state['step'] == 1).all() and not ora.state['error'].any()
+    assert (ora.state['cell'] != state['cell']).any() and (ora.done & K.OUT_VALID).all()
+
+
 def test_program_guard_reports_bad_agent_index():
     """An agent index outside [0, A) does nothing; the env records error 3 and reports ERROR | ALL_DONE, then auto-resets."""
     bad = DeviceProgram('BGWP_FN void bgwp_step(bgwp_ctx *c) { if (bgwp_step_index(c) == 2) bgwp_set_health(c, bgwp_n_agents(c), 0.5); }')
     sim = ForagingSim.build()
     sim.device_program = lambda: bad
     spec = compile_sim(sim, n_envs=4, seed=1, auto_reset=True)
-    ora = ProgramOracleEnv(spec)
+    ora = OracleEnv(spec)
     ora.reset()
     ora.step(ora.sample_actions())
     assert not (ora.all_done & K.ENV_ERROR).any() and not ora.state['error'].any()
@@ -226,7 +246,7 @@ def test_float_constant_round_trips_exactly():
     sim.device_program = lambda: program
     spec = compile_sim(sim, n_envs=1, seed=5)
     assert f'#define X ({x.hex()})' in spec.program_source
-    ora = ProgramOracleEnv(spec)
+    ora = OracleEnv(spec)
     ora.reset()
     act = ora.sample_actions()
     ora.step(act)
