@@ -49,6 +49,14 @@ struct DeviceGuard {
 int align16(int x) { return (x + 15) & ~15; }
 int pow2ceil(int x) { int p = 1; while (p < x) p <<= 1; return p; }
 
+/* persistent grid of the specialised kernel: the resident set (per_sm CTAs on each of sms SMs), at most one CTA per env;
+ * BGW_GRID=n runs n CTAs instead (tests: many envs per CTA) */
+int fast_grid_ctas(int E, int per_sm, int sms)
+{
+    if (const char *t = getenv("BGW_GRID")) { const int v = atoi(t); if (v >= 1) return std::min(E, v); }
+    return std::max(1, std::min(E, per_sm * sms));
+}
+
 }  // namespace
 
 static const void *observe_fast_fn(int R)
@@ -75,10 +83,8 @@ struct BgwEngine {
     DevSpec ds{}, dsf{};          /* general kernels / fast kernel (own slot table size) */
     FastSpec fs{};
     int threads_fast = 0;
-    bool pdl = true;              /* launch the fast step kernel with programmatic stream serialization */
     bool poisoned = false;        /* a step launch was rejected: the ticket counters are out of step */
     bool chain_ok = false;        /* consecutive launches of bgw_rollout_sampled may be chained per env (bgw_fast.cuh) */
-    bool rollout_fused = true;    /* bgw_rollout_sampled runs a rollout of the specialised kernel in one launch (BGW_ROLLOUT_FUSED=0: one launch per step) */
     bool randomize_action_input = false;   /* AllStepManager(randomize_action_input): steps without a caller-given order use the keyed one */
     int16_t *order_buf = nullptr;     /* [E][L] device: the keyed order of the step (bgw_order_kernel) */
     bool use_device_layouts = true;   /* bgw_use_device_layouts(): the caller supplies its own layouts when false */
@@ -495,7 +501,6 @@ int bgw_create(const BgwSpec *sp, int device, bgw_handle *out)
     cudaError_t ce;
     /* a user step program has no stock instantiation: its kernel comes from bgw_set_program */
     h->step_fn = d.program == BGW_PROG_USER ? nullptr : bgw_general_step_fn(d.program, d.attack_actor);
-    if (const char *t = getenv("BGW_ALL_IN_ONE_KERNEL")) if (atoi(t) && h->step_fn) h->step_fn = bgw_general_step_fn(-1, -1);
     if ((h->step_fn && (ce = cudaFuncSetAttribute(h->step_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, off)) != cudaSuccess) ||
         (h->fs.enabled && (ce = cudaFuncSetAttribute(h->fast_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, h->fs.smem_bytes)) != cudaSuccess) ||
         (ce = cudaFuncSetAttribute(bgw_reset_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, off)) != cudaSuccess ||
@@ -513,7 +518,6 @@ int bgw_create(const BgwSpec *sp, int device, bgw_handle *out)
             (ce = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device)) != cudaSuccess)
             return bail(fail(2, "bgw_create: observe kernel set-up: %s", cudaGetErrorString(ce)));
         h->observe_grid = std::max(1, std::min(d.E, per_sm * sms));
-        if (const char *t = getenv("BGW_OBSERVE_GRID")) { const int v = atoi(t); if (v >= 1) h->observe_grid = std::min(d.E, v); }
     }
     if (getenv("BGW_VERBOSE")) {
         if (h->observe_fn) fprintf(stderr, "[bgw] observe kernel: gather-only, view %d\n", h->fs.uniform_view);
@@ -526,14 +530,12 @@ int bgw_create(const BgwSpec *sp, int device, bgw_handle *out)
         if (ce != cudaSuccess ||
             (ce = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device)) != cudaSuccess)
             return bail(fail(2, "bgw_create: occupancy query: %s", cudaGetErrorString(ce)));
-        h->fs.grid_ctas = std::max(1, std::min(d.E, per_sm * sms));
+        h->fs.grid_ctas = fast_grid_ctas(d.E, per_sm, sms);
         if (getenv("BGW_PROF_FILE")) {
             void *pp = nullptr;
             if (cudaMalloc(&pp, (size_t)h->fs.grid_ctas * 8 * 16 * sizeof(long long)) == cudaSuccess) { h->allocs.push_back(pp); cudaMemset(pp, 0, (size_t)h->fs.grid_ctas * 8 * 16 * sizeof(long long)); h->fs.prof = (long long *)pp; }
         }
         if (getenv("BGW_VERBOSE")) fprintf(stderr, "[bgw] fast kernel: shape %s, T=%d smem=%d B/CTA, %d CTAs/SM x %d SMs, grid=%d, slots=%d\n", h->fast_shape == 1 ? "C5 (compile-time)" : h->fast_shape == 2 ? "C2 (compile-time)" : "run-time", h->threads_fast, h->fs.smem_bytes, per_sm, sms, h->fs.grid_ctas, h->dsf.slot_mask + 1);
-        if (const char *t = getenv("BGW_PDL")) h->pdl = atoi(t) != 0;
-        if (const char *t = getenv("BGW_GRID")) { const int v = atoi(t); if (v >= 1) h->fs.grid_ctas = std::min(d.E, v); }
         {   /* env tickets + per-env launch stamps (bgw_fast.cuh, "env tickets and chained launches") */
             void *pp = nullptr;
             const size_t nb = ((size_t)d.E + BGW_TICKET_RING) * sizeof(uint32_t);
@@ -544,9 +546,7 @@ int bgw_create(const BgwSpec *sp, int device, bgw_handle *out)
             h->fs.env_seq = (uint32_t *)pp + BGW_TICKET_RING;
         }
         /* chained launches: nothing may run between two steps (no layout kernel) */
-        h->chain_ok = h->pdl && !(h->maze_ok && sp->auto_reset);
-        if (const char *t = getenv("BGW_CHAIN")) if (!atoi(t)) h->chain_ok = false;
-        if (const char *t = getenv("BGW_ROLLOUT_FUSED")) h->rollout_fused = atoi(t) != 0;
+        h->chain_ok = !(h->maze_ok && sp->auto_reset);
         h->fs.wait_limit_ns = 10ull * 1000ull * 1000ull * 1000ull;
         if (const char *t = getenv("BGW_WAIT_LIMIT_MS")) { const long long v = atoll(t); if (v > 0) h->fs.wait_limit_ns = (unsigned long long)v * 1000000ull; }
     }
@@ -603,8 +603,7 @@ int bgw_specialize(bgw_handle h, const char *cache_dir)
     const int rc = bgwjit::driver().OccupancyMaxActiveBlocks(&per_sm, h->fast_jit.function, h->threads_fast, (size_t)h->fs.smem_bytes);
     if (rc || per_sm < 1) { bgwjit::driver().ModuleUnload(h->fast_jit.module); h->fast_jit = bgwjit::Kernel(); return fail(2, "bgw_specialize: occupancy query of the compiled kernel failed (%d)", rc); }
     CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
-    h->fs.grid_ctas = std::max(1, std::min(h->ds.E, per_sm * sms));
-    if (const char *t = getenv("BGW_GRID")) { const int v = atoi(t); if (v >= 1) h->fs.grid_ctas = std::min(h->ds.E, v); }
+    h->fs.grid_ctas = fast_grid_ctas(h->ds.E, per_sm, sms);
     h->fast_jit_on = true;
     if (getenv("BGW_VERBOSE")) fprintf(stderr, "[bgw] fast kernel compiled for this spec's shape: %d CTAs/SM, grid=%d\n", per_sm, h->fs.grid_ctas);
     return 0;
@@ -651,7 +650,7 @@ int bgw_bind_state(bgw_handle h, const BgwState *state)
         int per_sm = 0, sms = 0;
         CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, h->fast_fn, h->threads_fast, (size_t)h->fs.smem_bytes));
         CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
-        h->fs.grid_ctas = std::max(1, std::min(h->ds.E, per_sm * sms));
+        h->fs.grid_ctas = fast_grid_ctas(h->ds.E, per_sm, sms);
     }
     return 0;
 }
@@ -745,10 +744,10 @@ static int step_impl(bgw_handle h, const int8_t *actions, int8_t *sampled, const
          * CTAs of this one become resident as that one's CTAs retire and run their env-independent set-up (spec
          * tables, clean dense arrays) while its last envs finish; they read and write nothing of the step state
          * before griddepcontrol.wait, which returns once the previous grid has completed and its writes are visible.
-         * After any other stream operation the attribute changes nothing.  BGW_PDL=0 turns it off (A/B). */
+         * After any other stream operation the attribute changes nothing. */
         cudaLaunchAttribute pdl_attr[1];
         pdl_attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        pdl_attr[0].val.programmaticStreamSerializationAllowed = h->pdl ? 1 : 0;
+        pdl_attr[0].val.programmaticStreamSerializationAllowed = 1;
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3((unsigned)h->fs.grid_ctas); cfg.blockDim = dim3((unsigned)h->threads_fast);
         cfg.dynamicSmemBytes = (size_t)h->fs.smem_bytes; cfg.stream = (cudaStream_t)stream;
@@ -760,7 +759,7 @@ static int step_impl(bgw_handle h, const int8_t *actions, int8_t *sampled, const
             CUlaunchAttribute ja[1];
             memset(ja, 0, sizeof(ja));
             ja[0].id = CU_LAUNCH_ATTRIBUTE_PROGRAMMATIC_STREAM_SERIALIZATION;
-            ja[0].value.programmaticStreamSerializationAllowed = h->pdl ? 1 : 0;
+            ja[0].value.programmaticStreamSerializationAllowed = 1;
             CUlaunchConfig jc;
             memset(&jc, 0, sizeof(jc));
             jc.gridDimX = (unsigned)h->fs.grid_ctas; jc.gridDimY = jc.gridDimZ = 1;
@@ -831,7 +830,7 @@ int bgw_rollout_sampled(bgw_handle h, int n_steps, int8_t *actions_out, const in
             if (qe != cudaSuccess && qe != cudaErrorNotReady) { h->poisoned = true; return fail(2, "bgw_rollout_sampled: the stream reports %s; the handle cannot be used any more", cudaGetErrorString(qe)); }
         }
     }
-    if (h->fs.enabled && h->rollout_fused && !layouts_between && !(h->randomize_action_input && !order) && capture == cudaStreamCaptureStatusNone) {
+    if (h->fs.enabled && !layouts_between && !(h->randomize_action_input && !order) && capture == cudaStreamCaptureStatusNone) {
         /* the specialised kernel runs the whole rollout in ONE launch: its CTAs draw (step, env) tickets and an env's step
          * k + 1 starts as soon as its step k is stamped (bgw_fast.cuh); the per-CTA set-up is paid once per rollout */
         const int kmax = std::max(1, (int)(0x7FFFFFFFu / (uint32_t)h->ds.E) - 1);
@@ -841,8 +840,8 @@ int bgw_rollout_sampled(bgw_handle h, int n_steps, int8_t *actions_out, const in
         }
     } else {
         for (int i = 0; i < n_steps; ++i) {
-            /* launches 2..n follow a step launch of this handle directly: they may be chained per env */
-            const int rc = step_impl(h, nullptr, actions_out, order, obs, reward, done, all_done, stream, i > 0 && !layouts_between);
+            /* unchained: layouts run between steps, step_impl unchains the keyed order and capture, the general kernel never chains */
+            const int rc = step_impl(h, nullptr, actions_out, order, obs, reward, done, all_done, stream, false);
             if (rc) return rc;
             if (layouts_between) {                                 /* next episode's layouts of the envs that just finished */
                 const int rl = bgw_generate_layouts(h, nullptr, 1, stream);

@@ -450,19 +450,7 @@ __device__ __forceinline__ bool attack_holds(const DevSpec &s, const uint32_t *t
 /* The warp that runs the single-warp reservation rounds of an env: the LAST one; the first one compacts and keeps the books
  * (tickets, env flags, statistics).  With every single-warp job on warp 0 the sub-partitions that hold the first warps issued
  * 68 % of their slots and the others 38 %; measured with the rounds moved: 0.0423 -> 0.0408 ms per step (driver setting). */
-#ifdef BGW_ROUNDS_FIRST
-#define BGW_ROUNDS_WARP(T) 0
-#else
 #define BGW_ROUNDS_WARP(T) (((T) >> 5) - 1)
-#endif
-#ifndef BGW_BOOK_TID      /* the thread that closes an env's step: done test, env flags, statistics */
-#define BGW_BOOK_TID 0
-#endif
-#ifdef BGW_COMPACT_LAST
-#define BGW_COMPACT_WARP(T) (((T) >> 5) - 1)
-#else
-#define BGW_COMPACT_WARP(T) 0
-#endif
 
 template <bool WARP, typename HT>
 __device__ uint32_t fast_attack_rounds(const DevSpec &s, const FastSpec &f, Env &ev, FastEnv &fe, int n_eff, uint32_t epoch, int tid, int T)
@@ -856,14 +844,10 @@ __device__ void fast_obs_rows_lane(const DevSpec &s, const FastSpec &f, const En
                     if (d + n <= 64 * g || d >= 64 * (g + 1)) continue;   /* row does not touch this group */
                     const uint32_t *rp = wp + i * pw4;
                     uint32_t x[LW + 1], y[RW];
-#if defined(BGW_EXP_OBS1)          /* timing experiment only (wrong observations): one load per window row */
-#pragma unroll
-                    for (int j = 0; j < LW; ++j) x[j] = rp[0];
-#else                              /* the last aligned word only where the row reaches into it: a third of the gather's
-                                      shared-memory wavefronts are bank conflicts of 32 unrelated rows, fewer lanes, fewer conflicts */
+                    /* the last aligned word only where the row reaches into it: a third of the gather's shared-memory
+                       wavefronts are bank conflicts of 32 unrelated rows, fewer lanes, fewer conflicts */
 #pragma unroll
                     for (int j = 0; j < LW; ++j) x[j] = (j < LW - 1 || sh + 8 * n > 32 * (LW - 1)) ? rp[j] : 0u;
-#endif
                     x[LW] = 0;
 #pragma unroll
                     for (int j = 0; j < RW; ++j) y[j] = __funnelshift_r(x[j], x[j + 1], sh);
@@ -895,29 +879,20 @@ template <int R>
 __device__ __forceinline__ void fast_obs_rows(const DevSpec &s, const FastSpec &f, const Env &ev, const FastEnv &fe, int n_act, int8_t *obs_env,
                                               int tid, int T)
 {
-#ifndef BGW_OBS_ONE_LANE
     if constexpr (ObsCoop<R>::on) fast_obs_rows_coop<R>(s, f, ev, fe, n_act, obs_env, tid, T);
-    else
-#endif
-        fast_obs_rows_lane<R>(s, f, ev, fe, n_act, obs_env, tid, T);
+    else fast_obs_rows_lane<R>(s, f, ev, fe, n_act, obs_env, tid, T);
 }
 
 /* Compile-time shape of the headline workload (BASELINE configs[4]: 64x64 grid, 256 agents that are all learners,
  * view 5, MoveActor, observe_self, OneTeamRemainingDone).  bgw_create selects the instantiation of a shape when the
  * compiled spec matches it exactly; every other sim runs the FastDynamic instantiation with run-time shapes.  The
  * code is the same: the constants below only let the compiler fold divisions, strides and trip counts. */
-#ifndef BGW_C5_LB_N
-#define BGW_C5_LB_N 8
-#endif
-#ifndef BGW_STATIC_T
-#define BGW_STATIC_T 64      /* threads per env of the compile-time-shape instantiation (A/B builds: -DBGW_STATIC_T=64 with BGW_THREADS=64) */
-#endif
 struct FastStaticC5 {
     static constexpr bool is_static = true;
     static constexpr int A = 256, L = 256, H = 64, W = 64, P = 5, PL = 5, PW = 76, PH = 74, obs_stride = 128, nchunks = 8,
                          obs_h = 11, view = 5, move_actor = BGW_MOVE_BOX, ravel = 0, observe_self = 1, done_mask = BGW_DONE_ONE_TEAM,
-                         max_enc = 4, simd_ok = 1, async_ok = 1, slots = 256, T = BGW_STATIC_T, att = 1, identity = 1, can_mix = 0, acc_lt1 = 0, rpo = 0,
-                         LB_T = BGW_STATIC_T, LB_N = BGW_C5_LB_N;
+                         max_enc = 4, simd_ok = 1, async_ok = 1, slots = 256, T = 64, att = 1, identity = 1, can_mix = 0, acc_lt1 = 0, rpo = 0,
+                         LB_T = 64, LB_N = 8;
 };
 /* BASELINE configs[1] (examples/rllib_team_battle.py: 8x8 grid, 24 agents in 4 teams, view 3): one warp per env, 32 envs
  * per SM, each at its own place in the code -- the run-time-shape instantiation (9.3 k instructions) spends most of its
@@ -971,8 +946,7 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
     }
     int T_ = (int)blockDim.x;
     if constexpr (SHAPE::is_static) T_ = SHAPE::T;
-    const int ptid = threadIdx.x, T = T_, lane = ptid & 31, nwarp = T >> 5;
-    int tid = ptid, warp = ptid >> 5;                      /* rotated per env inside the loop (below) */
+    const int tid = threadIdx.x, T = T_, lane = tid & 31, warp = tid >> 5, nwarp = T >> 5;
     unsigned char *scratch = bgw_smem + f.o_scratch;
     Env ev;
     ev.enc = (int8_t *)(bgw_smem + f.o_enc);
@@ -1069,46 +1043,22 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
     uint32_t epoch = f_in.epoch0;                         /* tag of the next reservation round (ordered rounds, above) */
     int it_no = -1, sl = 1;
     /* end of an env: hand the ticket drawn at its start to the next iteration, and once every thread's stores are
-     * behind a barrier, stamp the env (release: the barrier makes the other threads' stores cumulative) */
-#ifndef BGW_STAMP_TID     /* the thread that stamps: the fence of the release stalls its warp until the env's stores are performed, so it is
-                             a thread of the LAST warp, not of the warp that leads the env (measured: five episodes 0.0295 -> 0.0276 ms per step) */
-#define BGW_STAMP_TID (T - 1)
-#endif
-    /* -DBGW_STAMP_DEFERRED (A/B; measured SLOWER: five episodes 0.0272 -> 0.0288 ms per step, configs[1] 0.0299 -> 0.0317): write the
-     * stamp late -- at the emit phase of the CTA's next env, when the finished env's stores are long performed and the release's
-     * fence is free.  Deadlock-freedom then needs the pending stamp written before every blocking wait, at the end of the next
-     * env at the latest, and after the loop (all in place below).  What it costs: the env's next step finds the stamp missing
-     * more often when it looks ahead, and fetches late. */
-    int pend_e = -1;                                      /* (only ever set in the stamping thread) */
-    uint32_t pend_v = 0;
-#define BGW_FLUSH_STAMP()                                                            \
-    do {                                                                             \
-        if (pend_e >= 0) { st_release_u32(f_in.env_seq + pend_e, pend_v); pend_e = -1; } \
-    } while (0)
-#ifndef BGW_STAMP_DEFERRED
-#define BGW_STAMP_ENV() st_release_u32(f_in.env_seq + e, f_in.seq + (uint32_t)kstep)
-#else
-#define BGW_STAMP_ENV() do { pend_e = e; pend_v = f_in.seq + (uint32_t)kstep; } while (0)
-#endif
+     * behind a barrier, stamp the env (release: the barrier makes the other threads' stores cumulative).  Thread T - 1
+     * stamps: the fence of the release stalls its warp until the env's stores are performed, so the stamp is on the LAST
+     * warp, not on the warp that leads the env (measured: five episodes 0.0295 -> 0.0276 ms per step). */
 #define BGW_END_ENV()                                                                \
     do {                                                                             \
         if (tid == 0) tslot[sl ^ 1] = (int)tnew;                                     \
         __syncthreads();                                                             \
         BGW_JITTER_POINT(7);                                                         \
-        if (tid == BGW_STAMP_TID) { BGW_FLUSH_STAMP(); BGW_STAMP_ENV(); }            \
+        if (tid == T - 1) st_release_u32(f_in.env_seq + e, f_in.seq + (uint32_t)kstep); \
         sl ^= 1;                                                                     \
     } while (0)
     for (; g < NT; g = gn) {
         ++it_no;
-#ifdef BGW_WARP_ROTATION   /* measured: 0.0631 -> 0.0679 ms per step (slower); kept for A/B */
-        tid = ptid + 32 * (it_no % nwarp);
-        if (tid >= T) tid -= T;
-        warp = tid >> 5;
-#endif
         BGW_PROF_MARK(0);
         kstep = kn_carry; e = en_carry;                             /* (step, env) of this ticket: computed when it was `next` */
         if (late) {                                                 /* this ticket's rows were not ready when it was `next` */
-            BGW_FLUSH_STAMP();                                      /* (never block with a finished env unstamped) */
             env_wait_stamp(f_in, e, f_in.seq + (uint32_t)kstep - 1u);
             fast_issue_env(s, f, st, actions, e, bgw_smem + f.o_buf + b * f.buf_bytes, tid, T);
             ef_cur = __ldcg(&st.env_flags[e]); step_cur = __ldcg(&st.step[e]); epi_cur = __ldcg(&st.episode[e]);
@@ -1212,7 +1162,7 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
         /* ---- relevant entities and acting learners, both compacted in entity order ------------------ */
         int n_rel = 0, n_act = 0;
         if (f.simd_ok) {
-            if (warp == BGW_COMPACT_WARP(T)) {
+            if (warp == 0) {
                 const uint32_t *fw = (const uint32_t *)ev.flags, *kw = (const uint32_t *)ev.klass;
                 const int nwords = s.A >> 2, wpl = (nwords + 31) >> 5;
                 int cnt = 0;
@@ -1461,7 +1411,6 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
             if (pend) epoch = fast_move_phase<HT>(s, f, ev, fe, n_act, epoch, tid, T);
             BGW_PROF_MARK(8);
 
-            BGW_FLUSH_STAMP();                                      /* (BGW_STAMP_DEFERRED: the previous env's stores are long performed) */
             /* ---- entropy :58-59, rewards / dones of the acting learners (all_step_manager.py:68-87) -------- */
             for (int i = tid; i < n_act; i += T) {
                 const int a = ev.ragent[i], l = ev.plist[i];
@@ -1531,7 +1480,7 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
             }
         }
         __syncthreads();
-        if (tid == BGW_BOOK_TID && !fresh) {
+        if (tid == 0 && !fresh) {
             const unsigned long long encs = ((unsigned long long)(unsigned)ev.ctr[CTR_ENC_HI] << 32) | (unsigned)ev.ctr[CTR_ENC_LO];
             int d = !ev.ctr[CTR_AND];
             if (s.done_mask & BGW_DONE_ACTIVE) d &= (encs == 0);
@@ -1553,10 +1502,7 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
         BGW_END_ENV();                                              /* ctr, scratch and the staging buffer are rewritten next */
         BGW_PROF_MARK(11);
     }
-    BGW_FLUSH_STAMP();
 #undef BGW_END_ENV
-#undef BGW_STAMP_ENV
-#undef BGW_FLUSH_STAMP
     cp_async_wait<0>();
 }
 

@@ -590,7 +590,7 @@ def test_step_launch_replayed_from_a_cuda_graph(mirror):
 def test_chained_rollout_full_size_against_oracle(mirror):
     """The headline workload at full size (4096 envs: three envs per resident CTA, tickets, per-env stamps) through
     chained rollouts of several lengths, against the oracle on env slices at both ends of the batch, and against
-    serialised launches (BGW_CHAIN=0 semantics: step_sampled) over the whole batch."""
+    serialised launches (one unchained step_sampled per step) over the whole batch."""
     from abmarl_b200.engine import BatchedGridWorld
     from oracle.oracle import OracleEnv
     E, S = 4096, 6
