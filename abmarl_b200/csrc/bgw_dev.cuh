@@ -1399,9 +1399,8 @@ extern __shared__ __align__(16) unsigned char bgw_smem[];
 /* The library is built from three translation units so that they compile in parallel and a change to one kernel family
  * does not rebuild the others: bgw.cu (host side, small kernels), bgw_general.cu (bgw_step_kernel instantiations) and
  * bgw_fastk.cu (bgw_step_fast_kernel instantiations).  The kernel TUs hand their entry points to the host side: */
-typedef void (*GeneralStepFn)(const DevSpec, const BgwState, const uint32_t *, const int16_t *, int8_t *, float *, uint8_t *, uint8_t *);
 #ifndef __CUDACC_RTC__
-GeneralStepFn bgw_general_step_fn(int program, int attack_actor);   /* bgw_general.cu; (-1, -1) = every program and actor in one */
+const void *bgw_general_step_fn(int program, int attack_actor);      /* bgw_general.cu; (-1, -1) = every program and actor in one */
 const void *bgw_fast_step_fn(int shape, int head_elem);              /* bgw_fastk.cu; shape 0 run-time, 1 FastStaticC5, 2 FastStaticC2 */
 #endif
 

@@ -12,14 +12,13 @@
  *     #include "bgw_dev.cuh"
  *     extern "C" __global__ void bgw_step_jit(...) { bgw_step_body<PROG, ATT>(...); }
  *
- * for sm_100a into a cubin, which is loaded through the driver API (libcuda.so.1, dlopen) into the primary context the
- * runtime API uses, and launched with cuLaunchKernel.  bgw_set_program compiles the same kernel with a user step program
- * in it (bgw_program.cuh).  Host code only; included by bgw.cu.
+ * for sm_100a into a cubin, which the runtime loads as a library (cudaLibraryLoadData).  Its kernel, a cudaKernel_t cast to
+ * `const void *`, is set up and launched like a stock kernel.  bgw_set_program compiles the same kernel with a user step
+ * program in it (bgw_program.cuh).  Host code only; included by bgw.cu.
  */
 #ifndef BGW_JIT_H_
 #define BGW_JIT_H_
 
-#include <cuda.h>          /* types and constants only: the driver is opened with dlopen, nothing links against libcuda */
 #include <dlfcn.h>
 #include <sys/stat.h>
 
@@ -41,18 +40,6 @@ struct Nvrtc {
     const char *(*GetErrorString)(int) = nullptr;
     int (*Version)(int *, int *) = nullptr;
     int major = 0, minor = 0;
-};
-
-struct Driver {
-    void *lib = nullptr;
-    int (*ModuleLoadData)(CUmodule *, const void *) = nullptr;
-    int (*ModuleGetFunction)(CUfunction *, CUmodule, const char *) = nullptr;
-    int (*ModuleUnload)(CUmodule) = nullptr;
-    int (*FuncSetAttribute)(CUfunction, int, int) = nullptr;
-    int (*LaunchKernel)(CUfunction, unsigned, unsigned, unsigned, unsigned, unsigned, unsigned, unsigned, void *, void **, void **) = nullptr;
-    int (*LaunchKernelEx)(const CUlaunchConfig *, CUfunction, void **, void **) = nullptr;
-    int (*OccupancyMaxActiveBlocks)(int *, CUfunction, int, size_t) = nullptr;
-    int (*GetErrorString)(int, const char **) = nullptr;
 };
 
 template <typename F>
@@ -89,22 +76,7 @@ inline const char *load_nvrtc(Nvrtc &n)
     return nullptr;
 }
 
-inline const char *load_driver(Driver &d)
-{
-    if (d.lib) return nullptr;
-    if (!(d.lib = dlopen("libcuda.so.1", RTLD_NOW | RTLD_LOCAL))) return "libcuda.so.1 not found";
-    if (!sym(d.lib, "cuModuleLoadData", d.ModuleLoadData) || !sym(d.lib, "cuModuleGetFunction", d.ModuleGetFunction) ||
-        !sym(d.lib, "cuModuleUnload", d.ModuleUnload) || !sym(d.lib, "cuFuncSetAttribute", d.FuncSetAttribute) ||
-        !sym(d.lib, "cuLaunchKernel", d.LaunchKernel) || !sym(d.lib, "cuLaunchKernelEx", d.LaunchKernelEx) ||
-        !sym(d.lib, "cuOccupancyMaxActiveBlocksPerMultiprocessor", d.OccupancyMaxActiveBlocks) || !sym(d.lib, "cuGetErrorString", d.GetErrorString)) {
-        dlclose(d.lib); d.lib = nullptr;
-        return "libcuda.so.1 lacks an entry point";
-    }
-    return nullptr;
-}
-
 inline Nvrtc &nvrtc() { static Nvrtc n; return n; }
-inline Driver &driver() { static Driver d; return d; }
 
 /* directory of the shared object this code lives in (= abmarl_b200/csrc: the kernel sources sit next to libbgw.so) */
 inline std::string library_dir()
@@ -158,15 +130,14 @@ inline std::string pin_statements(const DevSpec &d, bool has_init_ammo)
 }
 
 struct Kernel {
-    CUmodule module = nullptr;
-    CUfunction function = nullptr;
+    cudaLibrary_t lib = nullptr;     /* owned by the caller: cudaLibraryUnload */
+    const void *fn = nullptr;        /* the cudaKernel_t, as the runtime's launch and attribute calls take it */
 };
 
 /* Compile `src` (or fetch its cubin from cache_dir) and load the kernel `name` with `smem` bytes of dynamic shared memory.
  * Returns nullptr on success, else a message (static or in `msg`). */
 inline const char *compile_and_load(std::string src, const char *name, int smem, const char *cache_dir, Kernel &out, std::string &msg)
 {
-    if (const char *e = load_driver(driver())) return e;
     const std::string dir = library_dir(), inc = dir + "/../../include";
     std::string dev, fst, prg, hdr, phl, sti, pgh;
     if (!read_file(dir + "/bgw_dev.cuh", dev) || !read_file(dir + "/bgw_fast.cuh", fst) || !read_file(dir + "/bgw_program.cuh", prg) ||
@@ -220,24 +191,23 @@ inline const char *compile_and_load(std::string src, const char *name, int smem,
                 }
             }
         }
-        Driver &c = driver();
-        const char *es = nullptr;
-        int rc = c.ModuleLoadData(&out.module, cubin.data());
-        if (!rc) {
-            rc = c.ModuleGetFunction(&out.function, out.module, name);
-            if (!rc) rc = c.FuncSetAttribute(out.function, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, smem);
-            if (!rc) break;
-            c.ModuleUnload(out.module);
+        cudaError_t rc = cudaLibraryLoadData(&out.lib, cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0);
+        if (rc == cudaSuccess) {
+            cudaKernel_t k = nullptr;
+            rc = cudaLibraryGetKernel(&k, out.lib, name);
+            if (rc == cudaSuccess) rc = cudaFuncSetAttribute((const void *)k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+            if (rc == cudaSuccess) { out.fn = (const void *)k; break; }
+            cudaLibraryUnload(out.lib);
         }
         out = Kernel();
+        cudaGetLastError();   /* the failure is reported here: step_impl's cudaPeekAtLastError must not take it for a failed launch */
         if (from_cache && attempt == 0) {                 /* a damaged or stale cache entry: compile afresh, once */
             from_cache = false;
             cubin.clear();
             remove(cache_path.c_str());
             continue;
         }
-        c.GetErrorString(rc, &es);
-        msg = std::string("loading ") + name + ": " + (es ? es : "?");
+        msg = std::string("cudaLibraryLoadData / cudaLibraryGetKernel of ") + name + ": " + cudaGetErrorString(rc);
         return msg.c_str();
     }
     return nullptr;
