@@ -919,6 +919,127 @@ inline bool fast_shape_matches(const DevSpec &q, const FastSpec &f, int threads)
 }
 #endif
 
+/* ---- phases of the per-env step (bgw_step_fast_body below), each run by every thread of the CTA ---------------------- */
+
+/* Occupant lists and summary of the relevant entities.  Entry: compaction.  Exit: head / cenc describe the grid, rflag and
+ * killrank of the relevant entities are clear (barrier). */
+template <typename HT>
+__device__ __forceinline__ void fast_build_lists(const DevSpec &s, const FastSpec &f, Env &ev, FastEnv &fe, int n_rel, int tid, int T)
+{
+    for (int x = tid; x < n_rel; x += T) {
+        const int a = fe.rel[x];
+        fe.rflag[a] = 0;
+        fe.killrank[a] = BGW_NONE16;
+        if (ev.flags[a] & BGW_ST_IN_GRID) {
+            if (ev.next[a] != BGW_NONE16) ev.tmp[ev.next[a]] = 1;
+            fe.cenc[pad_index(s, f, ev.cell[a])] = ev.enc[a];
+        }
+    }
+    __syncthreads();
+    for (int x = tid; x < n_rel; x += T) {
+        const int a = fe.rel[x];
+        if (ev.flags[a] & BGW_ST_IN_GRID) {
+            if (!ev.tmp[a]) ((HT *)fe.head)[ev.cell[a]] = (HT)a;
+            ev.tmp[a] = 0;
+            const int p = pad_index(s, f, ev.cell[a]);
+            if (f.can_mix && fe.cenc[p] != ev.enc[a]) { fe.cenc[p] = (int8_t)BGW_MIXED; ev.ctr[CTR_MIXED] = 1; }
+        }
+    }
+    __syncthreads();
+}
+
+/* Attack pre-pass (team_battle_example.py:35-47): each acting learner's learner index and action word, and for an attacker its
+ * candidate cells; an effective attacker (one with a possible victim) makes its first reservation under `epoch`.  Entry: the
+ * lists.  Exit: plist, act, rkmask, pstate and the effective attackers eff[0..ctr[CTR_NEMIT]) published (barrier). */
+__device__ __forceinline__ void fast_attack_prepass(const DevSpec &s, const FastSpec &f, Env &ev, FastEnv &fe, const uint32_t *actions,
+                                                    uint32_t *sampled, int n_act, uint32_t epoch, int tid, int T)
+{
+    const int e = ev.e;
+    for (int i = tid; i < n_act; i += T) {
+        const int a = ev.ragent[i], l = f.identity_learners ? a : __ldg(&s.learner_of[a]);
+        ev.plist[i] = (uint16_t)l;
+        if (sampled) {                                   /* bgw_step_sampled: the keyed random policy, fused */
+            const uint32_t w = sample_action_word(s, a, ev.klass[a], ev.genv, ev.episode, ev.step - 1u);
+            fe.act[l] = w;
+            sampled[(size_t)e * s.L + l] = w;
+        } else {
+            fe.act[l] = __ldcg(&actions[(size_t)e * s.L + l]);   /* (prefetched to L2 while the env before ran) */
+        }
+        uint8_t p = 0;
+        if ((ev.flags[a] & BGW_ST_ACTIVE) && (ev.klass[a] & BGW_AG_ATTACKING) && (int8_t)((fe.act[l] >> 16) & 0xFF) != 0) {
+            /* candidate cells: the summary says an attackable encoding (or a mix) is present */
+            const int R = f.uniform_att >= 0 ? f.uniform_att : __ldg(&s.attack_r[a]), n = 2 * R + 1;
+            const unsigned long long row = __ldg(&s.attack_map[ev.enc[a]]);
+            const int wo = pad_index(s, f, ev.cell[a]) - R * f.PW - R;
+            const int8_t *w = fe.cenc + wo;
+            uint32_t mask = 0;
+            if (R == 1) {
+                /* the three window rows as aligned word pairs, funnel-shifted to the window's first column; each of the nine
+                 * bytes is tested from the register: v in 1..max_enc selects its bit of the attack map row, 0 (empty) and -1
+                 * (border) select nothing (bit 0 of a row is never set; shifts clamp) */
+                const uint32_t *wp = reinterpret_cast<const uint32_t *>(fe.cenc + (wo & ~3));
+                const int sh = (wo & 3) * 8, pw4 = f.PW >> 2;
+                uint32_t y[3];
+#pragma unroll
+                for (int k = 0; k < 3; ++k) y[k] = __funnelshift_r(wp[k * pw4], wp[k * pw4 + 1], sh);
+                if (s.max_enc < 32) {
+                    const uint32_t row32 = (uint32_t)row & ~1u;
+#pragma unroll
+                    for (int k = 0; k < 9; ++k) {
+                        const uint32_t v = (y[k / 3] >> (8 * (k % 3))) & 0xFFu;
+                        mask |= (__funnelshift_rc(row32, 0u, v) & 1u) << k;
+                    }
+                } else {
+#pragma unroll
+                    for (int k = 0; k < 9; ++k) {
+                        const uint32_t v = (y[k / 3] >> (8 * (k % 3))) & 0xFFu;
+                        if (v < 64u && ((row >> v) & 1ull)) mask |= 1u << k;
+                    }
+                }
+                if (f.can_mix && ev.ctr[CTR_MIXED]) {           /* a mixed cell is always a candidate (the walk decides) */
+#pragma unroll
+                    for (int k = 0; k < 9; ++k)
+                        if (((y[k / 3] >> (8 * (k % 3))) & 0xFFu) == (uint32_t)(uint8_t)BGW_MIXED) mask |= 1u << k;
+                }
+            } else {
+                for (int wr = 0; wr < n; ++wr)
+                    for (int wc = 0; wc < n; ++wc) {
+                        const int v = w[wr * f.PW + wc];
+                        if (v > 0 ? (int)((row >> v) & 1ull) : (v == BGW_MIXED)) mask |= 1u << (wr * n + wc);
+                    }
+            }
+            fe.rkmask[i] = mask;
+            if (mask) {                                         /* effective attacker: first reservation right here */
+                p = 1; fe.eff[atomicAdd(&ev.ctr[CTR_NEMIT], 1)] = (uint16_t)i;
+                const SlotTables stt = slot_tables(s, ev);
+                attack_reserve(s, stt.t0, stt.mask, ev.cell[a], R, mask, (epoch << BGW_TAG_SHIFT) | (uint32_t)i);
+            }
+            else p = 3;                                         /* no possible victim: settled after the rounds */
+        }
+        ev.pstate[i] = p;
+    }
+    __syncthreads();
+}
+
+/* The ordered rounds of the effective attackers.  Entry: the attack pre-pass.  Exit: every attack executed (barrier when there
+ * was one); returns the next unused epoch, the same in every thread. */
+template <typename HT>
+__device__ __forceinline__ uint32_t fast_attack_phase(const DevSpec &s, const FastSpec &f, Env &ev, FastEnv &fe, uint32_t epoch, int lane, int warp, int T)
+{
+    const int n_eff = ev.ctr[CTR_NEMIT];
+    if (n_eff > 0) {          /* few agents (an attack action AND a possible victim next to them): one warp runs the rounds, also
+                                 beyond 32 of them; every thread keeps the same epoch */
+        if (warp == BGW_ROUNDS_WARP(T)) {
+            const uint32_t e2 = fast_attack_rounds<true, HT>(s, f, ev, fe, n_eff, epoch, lane, T);
+            if (lane == 0) ev.ctr[CTR_EPOCH] = (int)e2;
+        }
+        __syncthreads();
+        epoch = (uint32_t)ev.ctr[CTR_EPOCH];
+    }
+    else --epoch;
+    return epoch;
+}
+
 /* launch bounds per instantiation: the headline shape runs 64 threads per env and is limited to 11 envs per SM by shared memory,
  * so it may use more registers than the run-time-shape code (up to 128 threads): 71 instead of 64 makes its code 5 % smaller
  * (3568 instructions; measured +1 %) */
@@ -1264,27 +1385,7 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
         }
         BGW_PROF_MARK(3);
 
-        /* ---- occupant lists and summary from the relevant entities --------------------------------- */
-        for (int x = tid; x < n_rel; x += T) {
-            const int a = fe.rel[x];
-            fe.rflag[a] = 0;
-            fe.killrank[a] = BGW_NONE16;
-            if (ev.flags[a] & BGW_ST_IN_GRID) {
-                if (ev.next[a] != BGW_NONE16) ev.tmp[ev.next[a]] = 1;
-                fe.cenc[pad_index(s, f, ev.cell[a])] = ev.enc[a];
-            }
-        }
-        __syncthreads();
-        for (int x = tid; x < n_rel; x += T) {
-            const int a = fe.rel[x];
-            if (ev.flags[a] & BGW_ST_IN_GRID) {
-                if (!ev.tmp[a]) ((HT *)fe.head)[ev.cell[a]] = (HT)a;
-                ev.tmp[a] = 0;
-                const int p = pad_index(s, f, ev.cell[a]);
-                if (f.can_mix && fe.cenc[p] != ev.enc[a]) { fe.cenc[p] = (int8_t)BGW_MIXED; ev.ctr[CTR_MIXED] = 1; }
-            }
-        }
-        __syncthreads();
+        fast_build_lists<HT>(s, f, ev, fe, n_rel, tid, T);
         BGW_PROF_MARK(4);
 
         if (fresh) {
@@ -1293,85 +1394,9 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
              * which the compaction's barrier published) */
             if (!f.identity_learners) __syncthreads();
         } else {
-            /* ---- attack phase team_battle_example.py:35-47 ---------------------------------------------- */
-            for (int i = tid; i < n_act; i += T) {
-                const int a = ev.ragent[i], l = f.identity_learners ? a : __ldg(&s.learner_of[a]);
-                ev.plist[i] = (uint16_t)l;
-                if (sampled) {                                   /* bgw_step_sampled: the keyed random policy, fused */
-                    const uint32_t w = sample_action_word(s, a, ev.klass[a], ev.genv, ev.episode, ev.step - 1u);
-                    fe.act[l] = w;
-                    sampled[(size_t)e * s.L + l] = w;
-                } else {
-                    fe.act[l] = __ldcg(&actions[(size_t)e * s.L + l]);   /* (prefetched to L2 while the env before ran) */
-                }
-                uint8_t p = 0;
-                if ((ev.flags[a] & BGW_ST_ACTIVE) && (ev.klass[a] & BGW_AG_ATTACKING) && (int8_t)((fe.act[l] >> 16) & 0xFF) != 0) {
-                    /* candidate cells: the summary says an attackable encoding (or a mix) is present */
-                    const int R = f.uniform_att >= 0 ? f.uniform_att : __ldg(&s.attack_r[a]), n = 2 * R + 1;
-                    const unsigned long long row = __ldg(&s.attack_map[ev.enc[a]]);
-                    const int wo = pad_index(s, f, ev.cell[a]) - R * f.PW - R;
-                    const int8_t *w = fe.cenc + wo;
-                    uint32_t mask = 0;
-                    if (R == 1) {
-                        /* the three window rows as aligned word pairs, funnel-shifted to the window's first column; each
-                         * of the nine bytes is tested from the register: v in 1..max_enc selects its bit of the attack map
-                         * row, 0 (empty) and -1 (border) select nothing (bit 0 of a row is never set; shifts clamp) */
-                        const uint32_t *wp = reinterpret_cast<const uint32_t *>(fe.cenc + (wo & ~3));
-                        const int sh = (wo & 3) * 8, pw4 = f.PW >> 2;
-                        uint32_t y[3];
-    #pragma unroll
-                        for (int k = 0; k < 3; ++k) y[k] = __funnelshift_r(wp[k * pw4], wp[k * pw4 + 1], sh);
-                        if (s.max_enc < 32) {
-                            const uint32_t row32 = (uint32_t)row & ~1u;
-    #pragma unroll
-                            for (int k = 0; k < 9; ++k) {
-                                const uint32_t v = (y[k / 3] >> (8 * (k % 3))) & 0xFFu;
-                                mask |= (__funnelshift_rc(row32, 0u, v) & 1u) << k;
-                            }
-                        } else {
-    #pragma unroll
-                            for (int k = 0; k < 9; ++k) {
-                                const uint32_t v = (y[k / 3] >> (8 * (k % 3))) & 0xFFu;
-                                if (v < 64u && ((row >> v) & 1ull)) mask |= 1u << k;
-                            }
-                        }
-                        if (f.can_mix && ev.ctr[CTR_MIXED]) {           /* a mixed cell is always a candidate (the walk decides) */
-    #pragma unroll
-                            for (int k = 0; k < 9; ++k)
-                                if (((y[k / 3] >> (8 * (k % 3))) & 0xFFu) == (uint32_t)(uint8_t)BGW_MIXED) mask |= 1u << k;
-                        }
-                    } else {
-                        for (int wr = 0; wr < n; ++wr)
-                            for (int wc = 0; wc < n; ++wc) {
-                                const int v = w[wr * f.PW + wc];
-                                if (v > 0 ? (int)((row >> v) & 1ull) : (v == BGW_MIXED)) mask |= 1u << (wr * n + wc);
-                            }
-                    }
-                    fe.rkmask[i] = mask;
-                    if (mask) {                                         /* effective attacker: first reservation right here */
-                        p = 1; fe.eff[atomicAdd(&ev.ctr[CTR_NEMIT], 1)] = (uint16_t)i;
-                        const SlotTables stt = slot_tables(s, ev);
-                        attack_reserve(s, stt.t0, stt.mask, ev.cell[a], R, mask, (epoch << BGW_TAG_SHIFT) | (uint32_t)i);
-                    }
-                    else p = 3;                                         /* no possible victim: settled after the rounds */
-                }
-                ev.pstate[i] = p;
-            }
-            __syncthreads();
+            fast_attack_prepass(s, f, ev, fe, actions, sampled, n_act, epoch, tid, T);
             BGW_PROF_MARK(5);
-            {
-                const int n_eff = ev.ctr[CTR_NEMIT];
-                if (n_eff > 0) {          /* few agents (an attack action AND a possible victim next to them): one warp runs the
-                                             rounds, also beyond 32 of them; every thread keeps the same epoch */
-                    if (warp == BGW_ROUNDS_WARP(T)) {
-                        const uint32_t e2 = fast_attack_rounds<true, HT>(s, f, ev, fe, n_eff, epoch, lane, T);
-                        if (lane == 0) ev.ctr[CTR_EPOCH] = (int)e2;
-                    }
-                    __syncthreads();
-                    epoch = (uint32_t)ev.ctr[CTR_EPOCH];
-                }
-                else --epoch;
-            }
+            epoch = fast_attack_phase<HT>(s, f, ev, fe, epoch, lane, warp, T);
             BGW_PROF_MARK(6);
 
             /* ---- settle attackers without candidates; classify the moves :50-55 --------------------------- */
