@@ -25,7 +25,7 @@ OBS_POSITION_CENTERED, OBS_ABSOLUTE, OBS_STACKED = range(3)
 DONE_ACTIVE, DONE_ONE_TEAM, DONE_TARGET_AGENT, DONE_TARGET_DESTROYED = (1 << i for i in range(4))
 MANAGER_ALL_STEP, MANAGER_TURN_BASED, MANAGER_DYNAMIC_ORDER = range(3)
 RW_ATTACK_FAIL, RW_KILL, RW_DIE, RW_MOVE_FAIL, RW_ENTROPY, RW_TARGET, RW_EAT_FOOD = range(7)
-ST_ACTIVE, ST_IN_GRID, ST_DONE_REPORTED = 1, 2, 4
+ST_ACTIVE, ST_IN_GRID, ST_DONE_REPORTED, ST_NEXT = 1, 2, 4, 8
 ST_ORIENT_SHIFT = 4
 OUT_DONE, OUT_VALID = 1, 2
 ENV_ALL_DONE, ENV_RESET, ENV_TRUNCATED, ENV_ERROR = 1, 2, 4, 8

@@ -330,8 +330,6 @@ int check_spec(BgwEngine *h, const BgwSpec *sp, Plan &p)
     if (sp->program == BGW_PROG_REACH_TARGET && (d.a_target < 0 || learner_of[d.a_target] < 0))
         return fail(1, "bgw_create: ReachTheTargetSim needs a learning target agent");
     if (sp->program < BGW_PROG_TEAM_BATTLE || sp->program > BGW_PROG_USER) return fail(1, "bgw_create: unknown program %d", sp->program);
-    if (sp->program == BGW_PROG_USER && sp->manager == BGW_MANAGER_DYNAMIC_ORDER)
-        return fail(1, "bgw_create: a user step program cannot run under BGW_MANAGER_DYNAMIC_ORDER (its next_agent rule is built in)");
 
     int rc;
     std::vector<unsigned long long> ov(BGW_MAX_ENCODING + 1), am(BGW_MAX_ENCODING + 1);

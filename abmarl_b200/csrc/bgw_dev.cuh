@@ -904,6 +904,10 @@ static __device__ void user_step(const DevSpec &s, Env &ev, int nrank);
 static __device__ int user_done(const DevSpec &s, const Env &ev, int a);
 static __device__ int user_all_done(const DevSpec &s, const Env &ev);
 static __device__ double user_reward(const DevSpec &s, const Env &ev, int a, double acc);
+static __device__ int user_next_agent(const DevSpec &s, const Env &ev, int a);
+/* under BGW_MANAGER_DYNAMIC_ORDER: the size of this step's acting set (bgwp_n_acting) */
+enum { CTR_NACTING = CTR_EPOCH + 1 };
+static_assert(CTR_NACTING < CTR_COUNT, "ctr has no free slot");
 #endif
 
 /* sim.step(action_dict); ranks 0..nrank-1 hold the acting agents (ragent).  All threads, ends synchronised */
@@ -1514,7 +1518,27 @@ __device__ __forceinline__ void bgw_step_body(const DevSpec &s_in, const BgwStat
             const int a = __ldg(&s.agent_of[l]);
             ev.ragent[i] = (ev.flags[a] & BGW_ST_DONE_REPORTED) ? (uint16_t)BGW_NONE16 : (uint16_t)a;
         }
-    } else {                                                        /* turn_based_manager.py:46 */
+    }
+#ifdef BGW_USER_PROGRAM
+    else if (dynamic && s.program == BGW_PROG_USER) {              /* sim.next_agent of the previous step, in dict order */
+        if (tid == 0) {
+            int n = 0;
+            if (ev.step == 1u) {                                    /* reset named BgwState.turn (learner 0) */
+                const int a = __ldg(&s.agent_of[st.turn[e]]);
+                if (!(ev.flags[a] & BGW_ST_DONE_REPORTED)) ev.ragent[n++] = (uint16_t)a;
+            } else {
+                for (int l = 0; l < s.L; ++l) {
+                    const int a = __ldg(&s.agent_of[l]);
+                    if ((ev.flags[a] & (BGW_ST_NEXT | BGW_ST_DONE_REPORTED)) == BGW_ST_NEXT) ev.ragent[n++] = (uint16_t)a;
+                }
+            }
+            ev.ctr[CTR_NACTING] = n;
+        }
+        __syncthreads();
+        nrank = ev.ctr[CTR_NACTING];
+    }
+#endif
+    else {                                                          /* turn_based_manager.py:46 */
         nrank = 1;
         turn = st.turn[e];
         if (tid == 0) ev.ragent[0] = (uint16_t)__ldg(&s.agent_of[turn]);
@@ -1542,6 +1566,11 @@ __device__ __forceinline__ void bgw_step_body(const DevSpec &s_in, const BgwStat
         __syncthreads();
         if (tid == 0) ev.ctr[CTR_ENVDONE] = ev.ctr[CTR_ALLDONE] || ev.ctr[CTR_REMAINING] == 0;   /* :90-93 */
     } else {                                                        /* turn_based_manager.py:48-92 */
+#ifdef BGW_USER_PROGRAM
+        const bool named_by_program = dynamic && s.program == BGW_PROG_USER;
+        if (named_by_program && !ev.ctr[CTR_ALLDONE])              /* sim.next_agent: the hook for every learner (pstate is free after the step) */
+            for (int l = tid; l < s.L; l += T) ev.pstate[l] = (uint8_t)(user_next_agent(s, ev, __ldg(&s.agent_of[l])) > 0);
+#endif
         for (int l = tid; l < s.L; l += T) { dn[l] = 0; rew[l] = 0.f; }
         __syncthreads();
         if (tid == 0) {
@@ -1549,7 +1578,24 @@ __device__ __forceinline__ void bgw_step_body(const DevSpec &s_in, const BgwStat
             if (env_done) {                                         /* :49-57 (dynamic_order_manager.py:43-51 alike) */
                 for (int k = 0; k < s.L; ++k)
                     if (!(ev.flags[__ldg(&s.agent_of[k])] & BGW_ST_DONE_REPORTED)) ev.plist[ne++] = (uint16_t)k;
-            } else if (dynamic) {
+            }
+#ifdef BGW_USER_PROGRAM
+            else if (named_by_program) {                            /* dynamic_order_manager.py:52-85 over the named learners */
+                int next = -1;
+                for (int k = 0; k < s.L; ++k) {
+                    const int a = __ldg(&s.agent_of[k]);
+                    uint8_t f = ev.flags[a] & (uint8_t)~BGW_ST_NEXT;
+                    if (ev.pstate[k] && !(f & BGW_ST_DONE_REPORTED)) {
+                        ev.plist[ne++] = (uint16_t)k;
+                        if (prog_done(s, ev, a)) f |= BGW_ST_DONE_REPORTED;
+                        else { f |= BGW_ST_NEXT; if (next < 0) next = k; }
+                    }
+                    ev.flags[a] = f;
+                }
+                st.turn[e] = (int16_t)next;
+            }
+#endif
+            else if (dynamic) {
                 /* dynamic_order_manager.py:52-85 over next_agent = [the agent that acted, if this step finished it] + [the next
                  * agent in dict order that is not done] (examples: DynamicOrderMultiMazeSim.step) */
                 const int a0 = __ldg(&s.agent_of[turn]);

@@ -221,6 +221,8 @@ inline const char *build(const DevSpec &d, bool has_init_ammo, int threads, cons
     snprintf(head, sizeof(head), "#define BGW_JIT_T %d\n#define BGW_JIT_PIN ", threads);
     std::string src = std::string(program ? "#define BGW_USER_PROGRAM\n" : "") + head + pin_statements(d, has_init_ammo) +
                       "\n#include \"bgw_dev.cuh\"\n";
+    if (program && d.manager == BGW_MANAGER_DYNAMIC_ORDER)   /* the program's next_agent hook is required (bgw_program.cuh) */
+        src += "#define BGWP_DYNAMIC_ORDER\n";
     if (program)   /* the program's diagnostics name its own lines */
         src += std::string("#include \"bgw_program.cuh\"\n#line 1 \"program\"\n") + program +
                "\n#define BGWP_AFTER_PROGRAM\n#include \"bgw_program.cuh\"\n";

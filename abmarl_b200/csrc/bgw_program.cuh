@@ -8,7 +8,7 @@
  *     #include "bgw_program.cuh"        the API, ahead of the program
  *     <program source>
  *     #define BGWP_AFTER_PROGRAM
- *     #include "bgw_program.cuh"        user_step / user_done / ... : the engine's calls into the program
+ *     #include "bgw_program.cuh"        user_step / user_done / ... / user_next_agent: the engine's calls into the program
  *     <kernel wrapper>
  *
  * The program runs on thread 0 of the env's CTA between two barriers (prog_step), like the built-in serial programs,
@@ -34,7 +34,11 @@ static __device__ __forceinline__ bool bgwp_cell_ok(const bgwp_ctx *c, int r, in
 }
 
 /* ---- the acting set and the env ------------------------------------------------------------------------------------ */
-BGWP_FN int bgwp_n_acting(const bgwp_ctx *c) { return c->s->manager == BGW_MANAGER_ALL_STEP ? c->s->L : 1; }
+BGWP_FN int bgwp_n_acting(const bgwp_ctx *c)
+{
+    if (c->s->manager == BGW_MANAGER_DYNAMIC_ORDER) return c->ev->ctr[CTR_NACTING];
+    return c->s->manager == BGW_MANAGER_ALL_STEP ? c->s->L : 1;
+}
 BGWP_FN int bgwp_acting(const bgwp_ctx *c, int i)
 {
     if ((unsigned)i >= (unsigned)bgwp_n_acting(c)) { bgwp_fail(c); return -1; }
@@ -194,6 +198,22 @@ static __device__ double user_reward(const DevSpec &s, const Env &ev, int a, dou
 #else
     (void)s; (void)ev; (void)a;
     return acc;
+#endif
+}
+
+/* bgwjit::build defines BGWP_DYNAMIC_ORDER for a handle under BGW_MANAGER_DYNAMIC_ORDER: there the hook is the manager's rule */
+#if defined(BGWP_DYNAMIC_ORDER) && !defined(BGWP_HAS_NEXT_AGENT)
+#error "a step program under BGW_MANAGER_DYNAMIC_ORDER must define bgwp_next_agent (#define BGWP_HAS_NEXT_AGENT, include/bgw_program.h)"
+#endif
+
+static __device__ int user_next_agent(const DevSpec &s, const Env &ev, int a)
+{
+#ifdef BGWP_HAS_NEXT_AGENT
+    const bgwp_ctx c = {&s, const_cast<Env *>(&ev)};
+    return bgwp_next_agent(&c, a) != 0;
+#else
+    (void)s; (void)ev; (void)a;
+    return -1;
 #endif
 }
 

@@ -1,5 +1,6 @@
-"""Example simulations (definitions): the four sims named by the BASELINE configs, ReachTheTargetSim, and ForagingSim (a sim
-of its own that runs through a step program, abmarl_b200.program)."""
+"""Example simulations (definitions): the four sims named by the BASELINE configs, ReachTheTargetSim, ForagingSim (a sim
+of its own that runs through a step program, abmarl_b200.program) and AlternatingBattleSim (teams that take turns under the
+DynamicOrderManager, through a step program's next_agent hook)."""
 from .sims import (  # noqa: F401
     BattleAgent, TeamBattleSim,
     MazeNavigationAgent, MazeNavigationSim,
@@ -8,3 +9,4 @@ from .sims import (  # noqa: F401
     BarrierAgent, TargetAgent, RunningAgent, ReachTheTargetSim, TargetDone, OnlyAgentLeftDone,
 )
 from .foraging import Forager, Predator, Resource, ForagingSim  # noqa: F401,E402
+from .alternating_battle import AlternatingBattleSim  # noqa: F401,E402

@@ -207,9 +207,12 @@ class TurnBasedManager(SimulationManager):
 
 
 class DynamicOrderManager(SimulationManager):
-    """dynamic_order_manager.py:7-87: the simulation decides whose turn it is.  `actions[e, turn[e]]` is read; the step
-    reports the agents the simulation names next (the one that just finished, if any, and the next one that is not
-    done), or every agent not yet reported once the simulation is done."""
+    """dynamic_order_manager.py:7-87: the simulation decides whose turn it is.  `actions[e, l]` is read for every acting
+    learner (`acting`); the step reports the agents the simulation names next (sim.next_agent) that were not reported
+    done before, or every agent not yet reported once the simulation is done.  The built-in DynamicOrderMultiMazeSim names
+    the one that just finished, if any, and the next one that is not done: one learner acts, `turn[e]`.  A sim with a
+    device program names its agents with the program's next_agent hook (include/bgw_program.h): any number of learners
+    act at once, in dict order."""
     _manager = 'dynamic_order'
 
     def __init__(self, sim, **kwargs):
@@ -220,6 +223,22 @@ class DynamicOrderManager(SimulationManager):
 
     @property
     def turn(self):
-        """int16 [E]: the learner whose action the next step() consumes (the not-done agent the simulation named)."""
+        """int16 [E]: the learner whose action the next step() consumes (the not-done agent the simulation named); with a
+        device program the lowest such learner, -1 if it named none."""
         return self.engine.state['turn']
+
+    @property
+    def acting(self):
+        """bool [E, L] on the device: the learners whose action rows the next step() reads.  After a reset that is
+        learner `turn[e]`; after a step, the learners the simulation named that are not done.  Learners already reported
+        done never act, and nobody acts in an env whose episode is over (the next step resets it)."""
+        st = self.engine.state
+        flags = st['flags'][:, self.spec.learner_agents]
+        by_turn = torch.arange(self.engine.L, device=flags.device)[None, :] == st['turn'].long()[:, None]
+        if self.spec.program == K.PROG_USER:
+            named = torch.where((st['step'] == 0)[:, None], by_turn, (flags & K.ST_NEXT) != 0)
+        else:
+            named = by_turn
+        live = (st['env_flags'] & K.ENV_ALL_DONE) == 0
+        return named & ((flags & K.ST_DONE_REPORTED) == 0) & live[:, None]
 

@@ -182,7 +182,8 @@ class AgentBasedSimulation(ABC):
 
 class DynamicOrderSimulation(AgentBasedSimulation):
     """agent_based_simulation.py:297-317: an AgentBasedSimulation where the simulation chooses the agents' turns
-    dynamically.  On the device the choice is part of the step kernel (BGW_MANAGER_DYNAMIC_ORDER, include/bgw.h); this
+    dynamically.  On the device the choice is part of the step kernel (BGW_MANAGER_DYNAMIC_ORDER, include/bgw.h): built in for
+    DynamicOrderMultiMazeSim, a step program's next_agent hook otherwise (include/bgw_program.h); this
     declaration keeps the reference's property for host-side code that inspects it."""
 
     @property

@@ -8,6 +8,7 @@ objects built by the unmodified reference (used when generating the golden vecto
 """
 import ctypes as C
 import math
+import re
 
 import numpy as np
 
@@ -142,14 +143,19 @@ def compile_sim(sim, manager='all_step', n_envs=1, env_offset=0, seed=0, horizon
         if not isinstance(program, DeviceProgram):
             raise TypeError(f"{type(sim).__name__}.device_program() must return an abmarl_b200.program.DeviceProgram")
         if manager == 'dynamic_order':
-            raise ValueError("a device program cannot run under the DynamicOrderManager: its next_agent rule is not programmable")
+            # the program's next_agent hook is the manager's rule (include/bgw_program.h)
+            if 'DynamicOrderSimulation' not in names:
+                raise ValueError("To use the DynamicOrderManager, the simulation must be a DynamicOrderSimulation.")
+            if not re.search(r'^\s*#\s*define\s+BGWP_HAS_NEXT_AGENT\b', program.assemble(sim.agents), re.MULTILINE):
+                raise ValueError("a device program under the DynamicOrderManager must define the next_agent hook "
+                                 "(#define BGWP_HAS_NEXT_AGENT, BGWP_FN int bgwp_next_agent(const bgwp_ctx *c, int a))")
         sp.program = K.PROG_USER
     else:
         sp.program = _first(names, _PROGRAMS, 'simulation class')
     sp.manager = {'all_step': K.MANAGER_ALL_STEP, 'turn_based': K.MANAGER_TURN_BASED,
                   'dynamic_order': K.MANAGER_DYNAMIC_ORDER}[manager]
-    if sp.manager == K.MANAGER_DYNAMIC_ORDER:
-        # the sim's next_agent rule runs on the device; the one rule built is DynamicOrderMultiMazeSim's (include/bgw.h)
+    if sp.manager == K.MANAGER_DYNAMIC_ORDER and program is None:
+        # the sim's next_agent rule runs on the device; the one rule built in is DynamicOrderMultiMazeSim's (include/bgw.h)
         assert 'DynamicOrderSimulation' in names and 'MultiMazeNavigationSim' in names, \
             "To use the DynamicOrderManager, the simulation must be a DynamicOrderSimulation (built: DynamicOrderMultiMazeSim)."
     sp.rows, sp.cols = int(sim.grid.rows), int(sim.grid.cols)

@@ -104,7 +104,13 @@ enum { BGW_MANAGER_ALL_STEP = 0 /* all_step_manager.py */, BGW_MANAGER_TURN_BASE
        /* managers/dynamic_order_manager.py:7-87 over a DynamicOrderSimulation (sim/agent_based_simulation.py:297-317) whose
         * next_agent rule is: the agent that just acted if that step finished it (it expects its last observation), then
         * the next agent in dict order that is not done -- abmarl_b200.examples.DynamicOrderMultiMazeSim.  BgwState.turn
-        * holds the learner whose action the next step consumes. */
+        * holds the learner whose action the next step consumes.
+        * A step program (BGW_PROG_USER) names the next agents itself with its next_agent hook (include/bgw_program.h),
+        * evaluated for every learner after the step: the named learners not yet reported done receive (obs, reward,
+        * done), and those of them that are not done carry BGW_ST_NEXT and act in the next step, all at once, in dict
+        * order.  The first step after a reset acts with learner 0 (BgwState.turn = 0).  BgwState.turn is the lowest
+        * learner carrying BGW_ST_NEXT, -1 if none: a step with nobody acting still runs, and only get_all_done or the
+        * horizon ends the episode. */
        BGW_MANAGER_DYNAMIC_ORDER = 2 };
 
 /* reward constant slots (float64; values live in the user's sim, e.g. team_battle_example.py:42-59) */
@@ -124,6 +130,8 @@ enum {
     BGW_ST_ACTIVE = 1 << 0,        /* PrincipleAgent.active / HealthAgent: health > 0   agent.py:192-196 */
     BGW_ST_IN_GRID = 1 << 1,       /* entity is present in its cell's dict              grid.py:107-140  */
     BGW_ST_DONE_REPORTED = 1 << 2, /* member of SimulationManager.done_agents           all_step_manager.py:85-87 */
+    BGW_ST_NEXT = 1 << 3,          /* in sim.next_agent and not done: acts in the next step (step programs under
+                                      BGW_MANAGER_DYNAMIC_ORDER only; never set otherwise) */
     BGW_ST_ORIENT_SHIFT = 4        /* bits 4..6: orientation 1..4 (0 = none)            agent.py:344     */
 };
 
@@ -386,8 +394,9 @@ int bgw_specialize(bgw_handle h, const char *cache_dir);
  * program and when the handle has a program already.  Until a program is set, bgw_reset, bgw_observe, bgw_sample_actions
  * and bgw_gather_valid work (they do not depend on the program) and bgw_step / bgw_step_sampled / bgw_rollout_sampled fail
  * without touching any buffer.  A program handle never runs the specialised team-battle kernel, and bgw_specialize on it
- * does nothing (the program's kernel is compiled for the spec already).  BGW_MANAGER_DYNAMIC_ORDER is not available to
- * programs (its next_agent rule is not programmable).
+ * does nothing (the program's kernel is compiled for the spec already).  Under BGW_MANAGER_DYNAMIC_ORDER the program must
+ * define the next_agent hook (BGWP_HAS_NEXT_AGENT, include/bgw_program.h); a program without it fails to compile here,
+ * with the reason in bgw_last_error().
  */
 int bgw_set_program(bgw_handle h, const char *source, const char *cache_dir);
 

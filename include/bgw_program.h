@@ -20,6 +20,16 @@
  *               acc is the reward accumulated for `a` since its last report (self.rewards[id], smart.py:101-104); the
  *               value returned is what the manager reports (e.g. multi_maze_navigation.py:56-59).  The accumulator is
  *               cleared after the report either way.
+ *     #define BGWP_HAS_NEXT_AGENT     BGWP_FN int bgwp_next_agent(const bgwp_ctx *c, int a)
+ *               1: agent a is in sim.next_agent after this step (DynamicOrderSimulation, agent_based_simulation.py:
+ *               297-317).  Required under the DynamicOrderManager, ignored under the other managers, so one program can
+ *               serve all three.  Evaluated for every learner, in parallel, after bgwp_step and get_all_done, on the
+ *               post-step state and only when get_all_done is false; bgwp_n_acting / bgwp_acting / bgwp_step_index still
+ *               describe the step just run ("the agent after the last one that acted" can be written).  Each named learner
+ *               not yet reported done receives (obs, reward, done); those of them that are not done act in the next step.
+ *               Limits: the named agents act together, in dict order (not in the order a next_agent list would give);
+ *               reset names learner 0, always (a program cannot choose the reset's next_agent: bgw_reset runs the stock
+ *               kernel).  A step that names nobody leaves the env stepping with no actor until get_all_done or the horizon.
  *   A hook that is not defined follows the SmartGridWorldSimulation rule over the spec's done components (smart.py:106-120:
  *   all() over them, so with none at all every agent is done) and reports the accumulator as it is.  The hooks take a const context: they may be
  *   evaluated on any thread, any number of times, so they must only read.  Every function that changes the simulation
@@ -53,11 +63,14 @@ typedef struct bgwp_ctx bgwp_ctx;
 BGWP_FN void bgwp_step(bgwp_ctx *c);
 
 /* ---- the acting set and the env ------------------------------------------------------------------------------------ */
-/* number of acting slots: the learners under AllStepManager, 1 under TurnBasedManager */
+/* number of acting slots: the learners under AllStepManager, 1 under TurnBasedManager; under DynamicOrderManager the learners
+ * bgwp_next_agent named after the previous step (learner 0 on the first step of an episode) that were not reported done,
+ * possibly 0 */
 BGWP_FN int bgwp_n_acting(const bgwp_ctx *c);
 /* agent of acting slot i in the order the manager hands the actions over (dict order, the caller's `order`, the keyed order
- * of randomize_action_input, all_step_manager.py:59-66; the learner whose turn it is, turn_based_manager.py:46), or -1 when
- * that learner was already reported done and sent no action (all_step_manager.py:59-61) */
+ * of randomize_action_input, all_step_manager.py:59-66; the learner whose turn it is, turn_based_manager.py:46; dict order
+ * under DynamicOrderManager, whatever `order` says), or -1 when that learner was already reported done and sent no action
+ * (all_step_manager.py:59-61) */
 BGWP_FN int bgwp_acting(const bgwp_ctx *c, int i);
 BGWP_FN int bgwp_step_index(const bgwp_ctx *c);   /* number of this step in the episode: 1 on the first step after a reset */
 BGWP_FN int bgwp_rows(const bgwp_ctx *c);         /* Grid.rows grid.py:20 */

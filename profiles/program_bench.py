@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """What a step program costs: agent-steps/s of one sim through a user step program against the built-in kernels.
 
-    python profiles/program_bench.py [--envs 16384] [--steps 200] [--warmup 20] [--out FILE.jsonl] [--repeat N]
+    python profiles/program_bench.py [--envs 16384] [--steps 200] [--warmup 20] [--out FILE.jsonl] [--repeat N] [--rows LABEL ...]
 
 Rows (16384 envs, keyed random policy, device-resident rollout through bgw_rollout_sampled, CUDA-event timing after a
 warm-up rollout; auto-reset, horizon 200):
@@ -10,6 +10,8 @@ warm-up rollout; auto-reset, horizon 200):
   tb_c2/general_specialized  ... after bgw_specialize
   tb_c2/default            the kernel bgw_create picks by default (the specialised team-battle kernel)
   foraging/program         abmarl_b200.examples.ForagingSim (ForagingSim.build(): 12x12, 6 foragers, 2 predators, 10 resources)
+  alternating_battle/program  abmarl_b200.examples.AlternatingBattleSim under the DynamicOrderManager (build(): 10x10,
+                           2 teams of 4 that take turns, the next_agent hook)
 Every row carries the card's name and power limit; the program rows carry the NVRTC compile time.  --repeat N runs the
 list N times (alternating the kernels) to show the spread.
 """
@@ -26,6 +28,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from abmarl_b200 import _capi as K                      # noqa: E402
 from abmarl_b200.engine import BatchedGridWorld         # noqa: E402
+from abmarl_b200.examples.alternating_battle import AlternatingBattleSim   # noqa: E402
 from abmarl_b200.examples.foraging import ForagingSim   # noqa: E402
 from abmarl_b200.spec import compile_sim                # noqa: E402
 from tests import program_cases                         # noqa: E402
@@ -78,7 +81,8 @@ def engines(n_envs):
             ('tb_c2/general', lambda: general(False)),
             ('tb_c2/general_specialized', lambda: general(True)),
             ('tb_c2/default', lambda: (BatchedGridWorld(base, device='cuda:0'), None)),
-            ('foraging/program', lambda: program(compile_sim(ForagingSim.build(), **kw)))]
+            ('foraging/program', lambda: program(compile_sim(ForagingSim.build(), **kw))),
+            ('alternating_battle/program', lambda: program(compile_sim(AlternatingBattleSim.build(), manager='dynamic_order', **kw)))]
 
 
 def main():
@@ -88,12 +92,13 @@ def main():
     ap.add_argument('--warmup', type=int, default=20)
     ap.add_argument('--repeat', type=int, default=1)
     ap.add_argument('--out', default=None)
+    ap.add_argument('--rows', nargs='*', default=None, help='labels of the rows to run (default: all)')
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("program_bench.py measures on a CUDA device; there is none")
     info = card()
     out = open(args.out, 'a') if args.out else None
-    rows = engines(args.envs)
+    rows = [r for r in engines(args.envs) if not args.rows or r[0] in args.rows]
     built = {}
     for rep in range(args.repeat):
         for label, make in rows:
