@@ -67,7 +67,7 @@ class BgwDims(C.Structure):
 
 LAYOUT_POSITION_STATE, LAYOUT_MAZE, LAYOUT_TARGET_BARRIERS_FREE = range(3)
 
-EXPORTS = ('bgw_create', 'bgw_destroy', 'bgw_dims', 'bgw_bind_state', 'bgw_reset', 'bgw_observe', 'bgw_specialize', 'bgw_set_program', 'bgw_step', 'bgw_generate_layouts',
+EXPORTS = ('bgw_create', 'bgw_destroy', 'bgw_dims', 'bgw_bind_state', 'bgw_reset', 'bgw_observe', 'bgw_specialize', 'bgw_set_program', 'bgw_set_program_vars', 'bgw_step', 'bgw_generate_layouts',
            'bgw_maze_layout_host', 'bgw_use_device_layouts',
            'bgw_sample_actions', 'bgw_step_sampled', 'bgw_rollout_sampled', 'bgw_gather_valid', 'bgw_rng_draw', 'bgw_los_mask', 'bgw_launch_count', 'bgw_last_error',
            'bgw_abi_version')
@@ -105,6 +105,8 @@ def load():
     lib.bgw_specialize.restype = C.c_int
     lib.bgw_set_program.argtypes = [h, C.c_char_p, C.c_char_p]
     lib.bgw_set_program.restype = C.c_int
+    lib.bgw_set_program_vars.argtypes = [h, C.c_int, C.c_int, _p, _p]
+    lib.bgw_set_program_vars.restype = C.c_int
     lib.bgw_step_sampled.argtypes = [h, _p, _p, _p, _p, _p, _p, _p]
     lib.bgw_step_sampled.restype = C.c_int
     lib.bgw_rollout_sampled.argtypes = [h, C.c_int, _p, _p, _p, _p, _p, _p, _p]

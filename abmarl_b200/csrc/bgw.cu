@@ -101,6 +101,8 @@ struct BgwEngine {
     KernelLaunch fast;            /* bgw_step_fast_kernel of this sim's shape, or compiled with this spec's shape (bgw_specialize) */
     KernelLaunch observe;         /* bgw_observe_fast_kernel<view range> when the sim qualifies, else the general observe kernel */
     KernelLaunch reset;
+    KernelLaunch program_vars;    /* bgw_program_vars_kernel: the initial values of the program's variables, after the reset kernel */
+    ProgVars pv{};                /* the step program's variables (bgw_set_program_vars); all 0 without */
     cudaLibrary_t jit = nullptr;  /* the library of the kernel bgw_specialize / bgw_set_program compiled (step.fn or fast.fn) */
     MazeParams maze{};            /* device-side MazePlacementState (bgw_maze.cuh); device pointers */
     bool maze_ok = false, maze_small = false;
@@ -216,12 +218,23 @@ MazeParams maze_params(const BgwSpec *sp, int max_enc)
     return m;
 }
 
+/* Let `fn` launch with `smem` bytes of dynamic shared memory.  The limit belongs to the kernel, not to a handle, and the stock
+ * kernels are shared by every handle of the process: it is only ever raised, so that creating a handle with a smaller working
+ * set does not make the launches of a larger one fail. */
+cudaError_t allow_smem(const void *fn, int smem)
+{
+    cudaFuncAttributes fa;
+    cudaError_t ce = cudaFuncGetAttributes(&fa, fn);
+    if (ce == cudaSuccess && fa.maxDynamicSharedSizeBytes < smem) ce = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    return ce;
+}
+
 /* Make `fn` the team-battle kernel step_impl launches: its dynamic shared memory, and the persistent grid of what fits the
  * device (per_sm: CTAs per SM).  On a failure the handle keeps the kernel it had, and the error is cleared so that
  * step_impl's cudaPeekAtLastError does not take it for a failed launch. */
 int use_fast_kernel(BgwEngine *h, const void *fn, int &per_sm)
 {
-    cudaError_t ce = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, h->fast.smem);
+    cudaError_t ce = allow_smem(fn, h->fast.smem);
     if (ce == cudaSuccess) ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, h->fast.threads, (size_t)h->fast.smem);
     if (ce != cudaSuccess || per_sm < 1) {
         cudaGetLastError();
@@ -481,7 +494,7 @@ int general_kernel(BgwEngine *h, const BgwSpec *sp, const Plan &p)
     h->step = {d.program == BGW_PROG_USER ? nullptr : bgw_general_step_fn(d.program, d.attack_actor), d.E, T, off, false};
     h->reset = {(const void *)bgw_reset_kernel, d.E, T, off, false};
     for (const KernelLaunch *k : {&h->step, &h->reset})
-        if (k->fn) CUDA_OK(cudaFuncSetAttribute(k->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, k->smem));
+        if (k->fn) CUDA_OK(allow_smem(k->fn, k->smem));
     return 0;
 }
 
@@ -553,7 +566,7 @@ int observe_kernel(BgwEngine *h, const BgwSpec *sp)
     const bool gather = f.enabled && !f.can_mix && sp->observe_self && f.uniform_view >= 1 && f.uniform_view <= 5 && !getenv("BGW_GENERIC_OBSERVE");
     if (gather) h->observe = {by_view[f.uniform_view], 0, 128, observe_layout(h->ds.A, h->ds.L, f.PH, f.PW).bytes, false};
     else h->observe = {(const void *)bgw_observe_kernel, h->ds.E, h->step.threads, h->step.smem, false};
-    CUDA_OK(cudaFuncSetAttribute(h->observe.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, h->observe.smem));
+    CUDA_OK(allow_smem(h->observe.fn, h->observe.smem));
     if (gather) {
         int per_sm = 0;
         CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, h->observe.fn, h->observe.threads, (size_t)h->observe.smem));
@@ -695,10 +708,30 @@ int bgw_set_program(bgw_handle h, const char *source, const char *cache_dir)
     if (!cache_dir) cache_dir = getenv("BGW_JIT_CACHE");
     std::string msg;
     bgwjit::Kernel k;
-    if (const char *e = bgwjit::build(h->ds, h->ds.init_ammo != nullptr, h->step.threads, cache_dir, k, msg, source))
+    if (const char *e = bgwjit::build(h->ds, h->ds.init_ammo != nullptr, h->step.threads, cache_dir, k, msg, source, h->pv))
         return fail(2, "bgw_set_program: %s", e);
     h->jit = k.lib;
     h->step.fn = k.fn;
+    return 0;
+}
+
+int bgw_set_program_vars(bgw_handle h, int n_env_vars, int n_agent_vars, const double *init, double *vars)
+{
+    if (!h) return fail(1, "bgw_set_program_vars: null handle");
+    if (h->ds.program != BGW_PROG_USER) return fail(1, "bgw_set_program_vars: the handle's spec runs built-in program %d, not BGW_PROG_USER", h->ds.program);
+    if (h->step.fn) return fail(1, "bgw_set_program_vars: the handle has a step program already (the counts are compiled into its kernel: call this first)");
+    if (n_env_vars < 0 || n_env_vars > BGW_MAX_ENV_VARS || n_agent_vars < 0 || n_agent_vars > BGW_MAX_AGENT_VARS)
+        return fail(1, "bgw_set_program_vars: %d env slots and %d agent variables, the limits are %d and %d", n_env_vars, n_agent_vars,
+                    BGW_MAX_ENV_VARS, BGW_MAX_AGENT_VARS);
+    const int stride = n_env_vars + h->ds.A * n_agent_vars;
+    if (stride && (!init || !vars)) return fail(1, "bgw_set_program_vars: init and vars are required for %d slots per env", stride);
+    DeviceGuard guard(h->device);
+    ProgVars pv{n_env_vars, n_agent_vars, stride, nullptr, stride ? vars : nullptr};
+    if (stride)
+        if (const int rc = upload(h, init, (size_t)stride, &pv.init)) return rc;
+    h->pv = pv;
+    const size_t n = (size_t)h->ds.E * stride;
+    h->program_vars = {(const void *)bgw_program_vars_kernel, (int)((n + 255) / 256), 256, 0, false};
     return 0;
 }
 
@@ -736,6 +769,11 @@ int bgw_reset(bgw_handle h, const uint8_t *env_mask, int8_t *obs, void *stream)
     void *args[] = {&h->ds, &h->st, &env_mask, &obs};
     if (const int rc = launch(h->reset, args, stream)) return rc;
     h->launches += 1;
+    if (h->pv.stride) {                                   /* the program's variables: the reset kernel is compiled without them */
+        void *vargs[] = {&h->pv, &h->ds.E, &env_mask};
+        if (const int rc = launch(h->program_vars, vargs, stream)) return rc;
+        h->launches += 1;
+    }
     return 0;
 }
 
@@ -819,7 +857,8 @@ static int step_impl(bgw_handle h, const int8_t *actions, int8_t *sampled, const
             actions = sampled;
         }
         const uint32_t *act_arg = (const uint32_t *)actions;
-        void *args[] = {&h->ds, &h->st, &act_arg, &order, &obs, &reward, &done, &all_done};
+        /* the kernel of a step program takes its variables last; the other kernels have eight parameters and ignore it */
+        void *args[] = {&h->ds, &h->st, &act_arg, &order, &obs, &reward, &done, &all_done, &h->pv};
         if (const int rc = launch(h->step, args, stream)) return rc;
     }
     h->launches += 1;

@@ -76,6 +76,16 @@ struct DevSpec {
         o_pstate, o_avail, o_mask, o_ctr, o_csum, smem_bytes;
 };
 
+/* A step program's variables (bgw_set_program_vars, include/bgw_program.h): one row of `stride` float64 per env in `vars`
+ * ([E][stride], caller-owned), the n_env env slots first, then [A][n_agent]; every reset writes `init` ([stride], device)
+ * into the row.  Only the program's kernel reads it, as a parameter of its own after all the others: every kernel takes
+ * DevSpec first, so a field appended to DevSpec would move each later parameter of every kernel. */
+struct ProgVars {
+    int n_env, n_agent, stride;
+    const double *init;
+    double *vars;
+};
+
 struct Env {
     uint16_t *head, *cell, *next, *ragent, *plist;
     uint32_t *slot, *act, *avail, *mask;
@@ -88,6 +98,10 @@ struct Env {
     int32_t *ammo;    /* this env's row of BgwState.ammo (global), or NULL */
     int e;
     uint32_t genv, episode, step;
+#ifdef BGW_USER_PROGRAM
+    ProgVars pv;      /* the program's variables (counts pinned at compile time) */
+    double *vars;     /* this env's row of pv.vars (global) */
+#endif
 };
 
 __device__ __forceinline__ void env_init(Env &ev, const DevSpec &s, unsigned char *sm)
@@ -1391,6 +1405,9 @@ static __device__ void env_reset(const DevSpec &s, const BgwState &st, Env &ev, 
             for (int it = tid; it < ne * s.nchunks; it += T)
                 *reinterpret_cast<uint4 *>(obs_env + (size_t)ev.plist[it / s.nchunks] * s.obs_stride + (it % s.nchunks) * 16) = make_uint4(0, 0, 0, 0);
     } else if (obs_env) observe_learners(s, ev, ne, obs_env, tid, T);
+#ifdef BGW_USER_PROGRAM
+    for (int j = tid; j < ev.pv.stride; j += T) ev.vars[j] = __ldg(&ev.pv.init[j]);   /* the program's variables (auto-reset) */
+#endif
     store_env(s, st, ev, true, tid, T);
     if (tid == 0) st.error[ev.e] = (uint32_t)ev.ctr[CTR_ERR];
 }
@@ -1420,6 +1437,16 @@ __global__ void bgw_reset_kernel(const DevSpec s, const BgwState st, const uint8
     ev.ammo = st.ammo ? st.ammo + (size_t)e * s.A : nullptr;
     env_reset(s, st, ev, obs ? obs + (size_t)e * s.L * s.obs_stride : nullptr, tid, T);
     if (tid == 0) st.env_flags[e] = (uint8_t)(ev.ctr[CTR_ERR] ? BGW_ENV_ERROR | BGW_ENV_ALL_DONE : 0);
+}
+
+/* The initial values of a step program's variables in the rows of the envs env_mask selects (NULL = all): bgw_reset runs it
+ * after bgw_reset_kernel, which is compiled without the program and knows nothing of them.  One thread per slot. */
+__global__ void bgw_program_vars_kernel(const ProgVars pv, int E, const uint8_t *env_mask)
+{
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)E * pv.stride) return;
+    if (env_mask && !env_mask[i / pv.stride]) return;
+    pv.vars[i] = __ldg(&pv.init[i % pv.stride]);
 }
 
 
@@ -1457,7 +1484,8 @@ __global__ void bgw_observe_kernel(const DevSpec s, const BgwState st, const uin
  * instantiation <-1, -1> is 26 k instructions (415 KB) and waits for instruction fetches most of the time. */
 template <int PROG, int ATT>
 __device__ __forceinline__ void bgw_step_body(const DevSpec &s_in, const BgwState &st, const uint32_t *actions, const int16_t *order,
-                                              int8_t *obs, float *reward, uint8_t *done, uint8_t *all_done)
+                                              int8_t *obs, float *reward, uint8_t *done, uint8_t *all_done,
+                                              ProgVars pv = ProgVars())   /* a step program's variables (its kernel only) */
 {
     DevSpec s = s_in;
     if (PROG >= 0) s.program = PROG;
@@ -1475,6 +1503,12 @@ __device__ __forceinline__ void bgw_step_body(const DevSpec &s_in, const BgwStat
     ev.e = e; ev.genv = (uint32_t)(s.env_offset + e);
     ev.health = st.health + (size_t)e * s.A;
     ev.ammo = st.ammo ? st.ammo + (size_t)e * s.A : nullptr;
+#ifdef BGW_USER_PROGRAM
+    ev.pv = pv;
+    ev.vars = pv.vars + (size_t)e * pv.stride;
+#else
+    (void)pv;
+#endif
     int8_t *obs_env = obs ? obs + (size_t)e * s.L * s.obs_stride : nullptr;
     float *rew = reward + (size_t)e * s.L;
     uint8_t *dn = done + (size_t)e * s.L;

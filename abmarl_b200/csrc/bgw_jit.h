@@ -107,8 +107,9 @@ inline unsigned long long fnv1a(const std::string &s, unsigned long long h = 146
     return h;
 }
 
-/* the statements that overwrite the spec's scalars at the top of bgw_step_body */
-inline std::string pin_statements(const DevSpec &d, bool has_init_ammo)
+/* the statements that overwrite the spec's scalars at the top of bgw_step_body; with `pv`, the counts of a step program's
+ * variables too (the code that touches them folds away when they are 0) */
+inline std::string pin_statements(const DevSpec &d, bool has_init_ammo, const ProgVars *pv = nullptr)
 {
     std::string s;
     char b[96];
@@ -126,6 +127,10 @@ inline std::string pin_statements(const DevSpec &d, bool has_init_ammo)
 #undef PIN
     if (!d.static_mask) s += "s.static_mask=nullptr;";
     if (!has_init_ammo) s += "s.init_ammo=nullptr;";
+    if (pv) {
+        snprintf(b, sizeof(b), "pv.n_env=%d;pv.n_agent=%d;pv.stride=%d;", pv->n_env, pv->n_agent, pv->stride);
+        s += b;
+    }
     return s;
 }
 
@@ -213,14 +218,15 @@ inline const char *compile_and_load(std::string src, const char *name, int smem,
     return nullptr;
 }
 
-/* the general step kernel for one spec; with `program` (a user step program, include/bgw_program.h) compiled into it */
+/* the general step kernel for one spec; with `program` (a user step program, include/bgw_program.h) compiled into it, with
+ * the counts of its variables `pv`, which the kernel takes as its last parameter */
 inline const char *build(const DevSpec &d, bool has_init_ammo, int threads, const char *cache_dir, Kernel &out, std::string &msg,
-                         const char *program = nullptr)
+                         const char *program = nullptr, const ProgVars &pv = ProgVars())
 {
     char head[1024];
     snprintf(head, sizeof(head), "#define BGW_JIT_T %d\n#define BGW_JIT_PIN ", threads);
-    std::string src = std::string(program ? "#define BGW_USER_PROGRAM\n" : "") + head + pin_statements(d, has_init_ammo) +
-                      "\n#include \"bgw_dev.cuh\"\n";
+    std::string src = std::string(program ? "#define BGW_USER_PROGRAM\n" : "") + head +
+                      pin_statements(d, has_init_ammo, program ? &pv : nullptr) + "\n#include \"bgw_dev.cuh\"\n";
     if (program && d.manager == BGW_MANAGER_DYNAMIC_ORDER)   /* the program's next_agent hook is required (bgw_program.cuh) */
         src += "#define BGWP_DYNAMIC_ORDER\n";
     if (program)   /* the program's diagnostics name its own lines */
@@ -228,9 +234,9 @@ inline const char *build(const DevSpec &d, bool has_init_ammo, int threads, cons
                "\n#define BGWP_AFTER_PROGRAM\n#include \"bgw_program.cuh\"\n";
     snprintf(head, sizeof(head),
              "extern \"C\" __global__ void __launch_bounds__(%d) bgw_step_jit(const DevSpec s_in, const BgwState st, const uint32_t *actions, "
-             "const int16_t *order, int8_t *obs, float *reward, uint8_t *done, uint8_t *all_done)\n"
-             "{ bgw_step_body<%d, %d>(s_in, st, actions, order, obs, reward, done, all_done); }\n",
-             threads, d.program, d.attack_actor);
+             "const int16_t *order, int8_t *obs, float *reward, uint8_t *done, uint8_t *all_done%s)\n"
+             "{ bgw_step_body<%d, %d>(s_in, st, actions, order, obs, reward, done, all_done%s); }\n",
+             threads, program ? ", const ProgVars pv" : "", d.program, d.attack_actor, program ? ", pv" : "");
     src += head;
     return compile_and_load(src, "bgw_step_jit", d.smem_bytes, cache_dir, out, msg);
 }

@@ -159,6 +159,25 @@ BGWP_FN double bgwp_uniform(const bgwp_ctx *c, int slot, int k)
     return bgw_u01(dev_draw(*c->s, *c->ev, BGW_SITE_PROGRAM, (uint32_t)slot, (uint32_t)k));
 }
 
+/* ---- the program's variables: the env's row of ProgVars.vars, in global memory like ev.health ------------------------ */
+BGWP_FN int bgwp_n_env_vars(const bgwp_ctx *c) { return c->ev->pv.n_env; }
+BGWP_FN int bgwp_n_agent_vars(const bgwp_ctx *c) { return c->ev->pv.n_agent; }
+static __device__ __forceinline__ double *bgwp_env_slot(const bgwp_ctx *c, int k)
+{
+    if ((unsigned)k >= (unsigned)c->ev->pv.n_env) { bgwp_fail(c); return nullptr; }
+    return c->ev->vars + k;
+}
+static __device__ __forceinline__ double *bgwp_agent_slot(const bgwp_ctx *c, int a, int k)
+{
+    if (!bgwp_agent_ok(c, a)) return nullptr;
+    if ((unsigned)k >= (unsigned)c->ev->pv.n_agent) { bgwp_fail(c); return nullptr; }
+    return c->ev->vars + c->ev->pv.n_env + a * c->ev->pv.n_agent + k;
+}
+BGWP_FN double bgwp_env_var(const bgwp_ctx *c, int k) { const double *p = bgwp_env_slot(c, k); return p ? __ldcg(p) : 0.0; }
+BGWP_FN void bgwp_set_env_var(bgwp_ctx *c, int k, double x) { if (double *p = bgwp_env_slot(c, k)) *p = x; }
+BGWP_FN double bgwp_agent_var(const bgwp_ctx *c, int a, int k) { const double *p = bgwp_agent_slot(c, a, k); return p ? __ldcg(p) : 0.0; }
+BGWP_FN void bgwp_set_agent_var(bgwp_ctx *c, int a, int k, double x) { if (double *p = bgwp_agent_slot(c, a, k)) *p = x; }
+
 #else  /* BGWP_AFTER_PROGRAM: the engine's calls into the program (bgw_dev.cuh declares them) */
 
 static __device__ void user_step(const DevSpec &s, Env &ev, int nrank)

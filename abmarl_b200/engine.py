@@ -44,6 +44,13 @@ class BatchedGridWorld:
         K.check(self.lib.bgw_create(C.byref(self._c), self.device.index, C.byref(h)), self.lib)
         self._h = h
         source = getattr(spec, 'program_source', None)
+        init = getattr(spec, 'program_var_init', None)
+        program_vars = None
+        if source is not None and init is not None:   # the program's variables: their counts are compiled into its kernel
+            program_vars = torch.zeros((spec.n_envs, init.size), dtype=torch.float64, device=self.device)
+            init = np.ascontiguousarray(init, dtype=np.float64)
+            K.check(self.lib.bgw_set_program_vars(h, spec.n_env_vars, len(spec.agent_var_names),
+                                                  init.ctypes.data_as(C.c_void_p), program_vars.data_ptr()), self.lib)
         if source is not None:                     # the sim's own step program, compiled into the step kernel (cached in $BGW_JIT_CACHE)
             K.check(self.lib.bgw_set_program(h, source.encode(), None), self.lib)
         d = K.BgwDims()
@@ -59,6 +66,7 @@ class BatchedGridWorld:
         self.state['episode'].fill_(-1)      # 0xFFFFFFFF: first reset makes it 0
         self.state['turn'].fill_(-1)
         self.state['stats'] = torch.zeros((self.E, K.BGW_STAT_COUNT), dtype=torch.int64, device=dev)
+        self.state['program_vars'] = program_vars    # float64 [E, n_env_vars + A * n_agent_vars] (program_vars()), or None
         # MazePlacementState: start layouts are generated on the device when the library can (bgw_generate_layouts),
         # else host-side (abmarl_b200/layouts.py) and handed over with set_layout()
         self.device_layouts = bool(d.device_layouts)
@@ -292,6 +300,14 @@ class BatchedGridWorld:
             if name in _NP_VIEW or name == 'stats':
                 a = a.view({2: np.int16, 4: np.int32, 8: np.int64}[a.dtype.itemsize])
             t.copy_(torch.from_numpy(a).reshape(t.shape))
+
+    def program_vars(self):
+        """{name: view} of the step program's variables in state['program_vars'] (DeviceProgram(env_vars=, agent_vars=)):
+        float64 [E] for an env scalar, [E, n] for an env array, [E, A] for an agent variable ({} without variables).
+        The obs rows do not carry them; these views are what a trainer reads, and what it writes is what the next
+        step reads."""
+        rows = self.state['program_vars']
+        return {} if rows is None else self.spec.program_var_views(rows)
 
     def stats(self):
         """Summed episode statistics (agent_steps, episodes, kills, env_steps) of this device's envs."""

@@ -100,6 +100,11 @@ class SimulationManager(ABC):
         snap['done'][env, l] = K.OUT_VALID
         return self.dicts_from(snap, env)[0][agent_id]
 
+    def program_vars(self):
+        """{name: view} of the device program's variables (BatchedGridWorld.program_vars): float64 [E] / [E, n] per env
+        variable, [E, A] per agent variable, on the device; {} for a sim without them."""
+        return self.engine.program_vars()
+
     def super_outputs(self):
         """SuperAgentWrapper view of the last step (super_agent_wrapper.py:112-216): (obs rows with null observations for
         covered agents done earlier, mask [E, L], reward [E, G] f64, done [E, G], valid [E, G]); groups = `super_view.groups`.

@@ -51,6 +51,11 @@ class CompiledSpec:
         self.agent_ids = []
         self.layout_generator = None     # e.g. ('maze', params) -> host-side layouts (abmarl_b200.layouts)
         self.program_source = None       # PROG_USER: the step program's C source (abmarl_b200.program, bgw_set_program)
+        # PROG_USER: the program's variables (bgw_set_program_vars): {name: (first slot, None | slots)}, the agent variables'
+        # names in slot order, and the float64 initial row [n_env_vars + n_agents * n_agent_vars] (None: no variables)
+        self.env_var_slots = {}
+        self.agent_var_names = []
+        self.program_var_init = None
 
     # ---- derived -----------------------------------------------------------------------------
     @property
@@ -79,6 +84,21 @@ class CompiledSpec:
             h = w = 2 * rmax + 1
         c = self.max_encoding if self.observer == K.OBS_STACKED else 1
         return h, w, c, (h * w * c + 15) // 16 * 16
+
+    @property
+    def n_env_vars(self):
+        return sum(1 if n is None else n for _, n in self.env_var_slots.values())
+
+    def program_var_views(self, rows):
+        """{name: view} of the program's variables in `rows` ([E, n_env_vars + n_agents * n_agent_vars], torch or numpy):
+        [E] for an env scalar, [E, n] for an env array, [E, A] for an agent variable."""
+        out = {}
+        for name, (k, n) in self.env_var_slots.items():
+            out[name] = rows[:, k] if n is None else rows[:, k:k + n]
+        per_agent = rows[:, self.n_env_vars:].reshape(rows.shape[0], self.n_agents, len(self.agent_var_names))
+        for k, name in enumerate(self.agent_var_names):
+            out[name] = per_agent[:, :, k]
+        return out
 
     def with_envs(self, n_envs, env_offset=0):
         import copy
@@ -282,6 +302,9 @@ def compile_sim(sim, manager='all_step', n_envs=1, env_offset=0, seed=0, horizon
     if sp.program == K.PROG_USER:               # the program carries its own constants and roles
         sp.program_source = program.assemble(sim.agents)
         sp.role[:] = program.role_table(sim.agents)
+        sp.env_var_slots, sp.agent_var_names = program.env_var_slots(), list(program.agent_vars)
+        if program.n_env_vars or program.n_agent_vars:
+            sp.program_var_init = np.array(program.var_init(sim.agents), dtype=np.float64)
     elif sp.program == K.PROG_TEAM_BATTLE:      # team_battle_example.py:42-59
         sp.reward[K.RW_ATTACK_FAIL] = rc.get('attack_fail', -0.1)
         sp.reward[K.RW_KILL] = rc.get('kill', 1.0)

@@ -42,6 +42,8 @@ extern "C" {
 #define BGW_NONE 0xFFFFu
 #define BGW_MAX_VICTIMS 256   /* attacked agents one attacker can name in one step (simultaneous_attacks x groups) */
 #define BGW_MAX_SIMATT 16     /* AttackingAgent.simultaneous_attacks                                             */
+#define BGW_MAX_ENV_VARS 65536  /* env slots of a step program's variables (bgw_set_program_vars)                  */
+#define BGW_MAX_AGENT_VARS 64   /* agent variables of a step program                                             */
 
 /* ---- per-agent class flags (which reference mixins the entity derives from) ------------------- */
 enum {
@@ -274,7 +276,8 @@ int bgw_bind_state(bgw_handle h, const BgwState *state);
  * AllStepManager.reset / TurnBasedManager.reset for the envs selected by env_mask ([E] u8 on device,
  * NULL = all): PositionState.reset, HealthState.reset, OrientationState.reset (state.py:88-166,629-641,
  * 666-675), rewards = 0 (smart.py:91), done_agents = non-learners (all_step_manager.py:41-44), then the
- * first observations into obs[E][L][obs_stride] (rows of unselected envs are untouched).
+ * first observations into obs[E][L][obs_stride] (rows of unselected envs are untouched).  A step program's variables
+ * (bgw_set_program_vars) get their initial values, by a second kernel after the reset's.
  */
 int bgw_reset(bgw_handle h, const uint8_t *env_mask, int8_t *obs, void *stream);
 
@@ -399,6 +402,21 @@ int bgw_specialize(bgw_handle h, const char *cache_dir);
  * with the reason in bgw_last_error().
  */
 int bgw_set_program(bgw_handle h, const char *source, const char *cache_dir);
+
+/*
+ * Declare the variables of a BGW_PROG_USER handle's step program (include/bgw_program.h) and bind their storage; call it
+ * before bgw_set_program, which compiles the counts into the program's kernel (they are part of its cache key):
+ *   n_env_vars    env slots, 0 .. BGW_MAX_ENV_VARS (a scalar takes one, an array one per element)
+ *   n_agent_vars  values per entity, 0 .. BGW_MAX_AGENT_VARS
+ *   init          HOST float64 [n_env_vars + A * n_agent_vars]: the initial row, env slots first, then [A][n_agent_vars];
+ *                 copied to the device here
+ *   vars          caller-owned DEVICE float64 [E][n_env_vars + A * n_agent_vars], env-major, like the BgwState arrays: every
+ *                 reset of an env (bgw_reset, auto-reset, one whose placement failed) writes `init` into its row; between
+ *                 resets only the program and the caller change it, and a value the caller writes is what the next step reads
+ * Fails on a handle of a built-in program, after bgw_set_program, on counts out of range, and on a null init or vars with
+ * a non-zero row.  A handle without variables runs exactly the kernels it runs without this call.
+ */
+int bgw_set_program_vars(bgw_handle h, int n_env_vars, int n_agent_vars, const double *init, double *vars);
 
 const char *bgw_last_error(void);
 int bgw_abi_version(void);

@@ -129,4 +129,19 @@ BGWP_FN void bgwp_add_reward(bgwp_ctx *c, int a, double x);
  * step; vary them to get independent draws.  Allowed in the hooks. */
 BGWP_FN double bgwp_uniform(const bgwp_ctx *c, int slot, int k);
 
+/* ---- the program's own variables ------------------------------------------------------------------------------------- */
+/* What a reference sim keeps on `self` and on its agents: float64 values of the program's own that persist from step to
+ * step.  Declared with DeviceProgram(env_vars=..., agent_vars=...) (abmarl_b200/program.py), which #defines each name as
+ * its index k (an env array: its first slot; slot i of it is NAME + i).  Env variables are slots 0 .. bgwp_n_env_vars(c) - 1,
+ * agent variables k = 0 .. bgwp_n_agent_vars(c) - 1 hold one value for each of the A entities.  Every reset of an env (an
+ * explicit one, an auto-reset, one whose placement failed) sets them to their declared initial values; otherwise only
+ * the program and the caller (who owns the buffer, bgw_set_program_vars in include/bgw.h) change them.  Reads are allowed
+ * in the hooks; writes take a non-const context.  An index out of range is bad input: 0.0, nothing written, error 3. */
+BGWP_FN int bgwp_n_env_vars(const bgwp_ctx *c);
+BGWP_FN int bgwp_n_agent_vars(const bgwp_ctx *c);
+BGWP_FN double bgwp_env_var(const bgwp_ctx *c, int k);
+BGWP_FN void bgwp_set_env_var(bgwp_ctx *c, int k, double x);
+BGWP_FN double bgwp_agent_var(const bgwp_ctx *c, int a, int k);
+BGWP_FN void bgwp_set_agent_var(bgwp_ctx *c, int a, int k, double x);
+
 #endif /* BGW_PROGRAM_H_ */

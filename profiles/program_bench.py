@@ -12,6 +12,8 @@ warm-up rollout; auto-reset, horizon 200):
   foraging/program         abmarl_b200.examples.ForagingSim (ForagingSim.build(): 12x12, 6 foragers, 2 predators, 10 resources)
   alternating_battle/program  abmarl_b200.examples.AlternatingBattleSim under the DynamicOrderManager (build(): 10x10,
                            2 teams of 4 that take turns, the next_agent hook)
+  king_of_the_hill/program abmarl_b200.examples.KingOfTheHillSim (build(): 10x10, 2 teams of 4, a 2x2 hill, target score 10,
+                           cooldown 2): a program with variables of its own (bgw_set_program_vars)
 Every row carries the card's name and power limit; the program rows carry the NVRTC compile time.  --repeat N runs the
 list N times (alternating the kernels) to show the spread.
 """
@@ -30,6 +32,7 @@ from abmarl_b200 import _capi as K                      # noqa: E402
 from abmarl_b200.engine import BatchedGridWorld         # noqa: E402
 from abmarl_b200.examples.alternating_battle import AlternatingBattleSim   # noqa: E402
 from abmarl_b200.examples.foraging import ForagingSim   # noqa: E402
+from abmarl_b200.examples.king_of_the_hill import KingOfTheHillSim   # noqa: E402
 from abmarl_b200.spec import compile_sim                # noqa: E402
 from tests import program_cases                         # noqa: E402
 
@@ -82,7 +85,8 @@ def engines(n_envs):
             ('tb_c2/general_specialized', lambda: general(True)),
             ('tb_c2/default', lambda: (BatchedGridWorld(base, device='cuda:0'), None)),
             ('foraging/program', lambda: program(compile_sim(ForagingSim.build(), **kw))),
-            ('alternating_battle/program', lambda: program(compile_sim(AlternatingBattleSim.build(), manager='dynamic_order', **kw)))]
+            ('alternating_battle/program', lambda: program(compile_sim(AlternatingBattleSim.build(), manager='dynamic_order', **kw))),
+            ('king_of_the_hill/program', lambda: program(compile_sim(KingOfTheHillSim.build(), **kw)))]
 
 
 def main():
