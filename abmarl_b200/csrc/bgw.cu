@@ -67,6 +67,23 @@ int fast_grid_ctas(int E, int per_sm, int sms)
     return std::max(1, std::min(E, per_sm * sms));
 }
 
+/* S, the consecutive steps of one env a ticket of the specialised kernel runs (bgw_fast.cuh, "env tickets and chained
+ * launches"), for a launch of K manager steps over E envs on `grid` resident CTAs.  Every step of a block after its first
+ * skips the env's hand-over (stamp wait, staging, list rebuild, write-back, summary clear, stamp), so a longer block is
+ * cheaper per step; but the launch ends with a tail of up to one block per CTA.  When the envs fit the resident CTAs each
+ * env is a serial chain anyway and has no tail to lengthen: the longest block.  Otherwise the block stays within a sixth
+ * of a CTA's share of the launch (K E / grid env-steps).  Measured on a B200 (profiles/r03_block_sweep.txt, S = 1..16):
+ * five episodes (K = 1000, share 2516) and configs[1] (K = 400, share 1384) are fastest at 16; K = 20 after a warm-up
+ * (share 50) at 8, and slower at 16. */
+int fast_block_steps(int K, int E, int grid)
+{
+    const long long share = (long long)K * E / std::max(grid, 1);
+    int S = 16;
+    if (E > grid)
+        while (S > 1 && S * 6LL > share) S >>= 1;
+    return std::max(1, std::min(S, K));
+}
+
 /* one kernel a handle launches, and how */
 struct KernelLaunch {
     const void *fn = nullptr;   /* a stock kernel, or the cudaKernel_t of one compiled at run time (bgw_jit.h) */
@@ -829,7 +846,9 @@ static int step_impl(bgw_handle h, const int8_t *actions, int8_t *sampled, const
         if (capture != cudaStreamCaptureStatusNone && n_steps != 1) return fail(1, "bgw_step: a captured launch is one manager step");
         h->fs.seq = h->seq + 1u;                       /* sequence number of this launch's first manager step */
         h->seq += (uint32_t)n_steps;
-        h->fs.n_tickets = (uint32_t)n_steps * (uint32_t)h->ds.E;
+        h->fs.n_steps = (uint32_t)n_steps;
+        h->fs.block_steps = (uint32_t)fast_block_steps(n_steps, h->ds.E, h->fast.grid);
+        h->fs.n_tickets = (uint32_t)((n_steps + h->fs.block_steps - 1) / h->fs.block_steps) * (uint32_t)h->ds.E;
         if (capture != cudaStreamCaptureStatusNone) {
             /* the launch goes into a CUDA graph and will run any number of times with these parameters: no ticket
              * counter (its base would be stale at the second replay) -- CTA c takes envs c, c + grid, ... -- and no
@@ -903,7 +922,7 @@ int bgw_rollout_sampled(bgw_handle h, int n_steps, int8_t *actions_out, const in
         }
     }
     if (h->fs.enabled && !layouts_between && !(h->randomize_action_input && !order) && capture == cudaStreamCaptureStatusNone) {
-        /* the specialised kernel runs the whole rollout in ONE launch: its CTAs draw (step, env) tickets and an env's step
+        /* the specialised kernel runs the whole rollout in ONE launch: its CTAs draw (block of steps, env) tickets and an env's step
          * k + 1 starts as soon as its step k is stamped (bgw_fast.cuh); the per-CTA set-up is paid once per rollout */
         const int kmax = std::max(1, (int)(0x7FFFFFFFu / (uint32_t)h->ds.E) - 1);
         for (int i = 0; i < n_steps; i += kmax) {

@@ -83,8 +83,10 @@ struct FastSpec {
                                  envs c, c + grid, ... (launches captured into a CUDA graph) */
     uint32_t ticket_base;     /* value of *ticket before this launch: every launch draws exactly n_tickets + grid tickets */
     uint32_t seq;             /* sequence number of the first manager step of this launch (1, 2, ... per handle) */
-    uint32_t n_tickets;       /* manager steps in this launch x E: ticket g is step g / E of env g % E (bgw_rollout_sampled runs a
-                                 whole rollout in ONE launch; bgw_step / bgw_step_sampled: E) */
+    uint32_t n_steps;         /* manager steps in this launch, K (bgw_rollout_sampled runs a whole rollout in ONE launch;
+                                 bgw_step / bgw_step_sampled: 1) */
+    uint32_t block_steps;     /* S: one ticket runs the consecutive steps [b S, min((b + 1) S, K)) of one env (fast_block_steps) */
+    uint32_t n_tickets;       /* ceil(K / S) x E: ticket g is block g / E of env g % E */
     unsigned long long wait_limit_ns;   /* longest legitimate wait for an env's stamp (env_wait_stamp) */
     int chain;                /* 1: the previous operation on the stream is the fast step launch seq - 1 of the same
                                  rollout (bgw_rollout_sampled): wait per env on env_seq, not for the whole grid */
@@ -274,9 +276,14 @@ template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile(
  * CTA only ever waits for envs that started or finished CTAs of the launch before own: the chain cannot deadlock.
  * Any number of launches can be in flight (a CTA of k that drew an expensive env -- one that resets -- is still
  * running while k+1, k+2, ... pass by, each leaving one CTA waiting for that env), at most one per resident CTA:
- * each launch has its own ticket counter in a ring of BGW_TICKET_RING > resident CTAs.  A launch draws exactly E
- * tickets (E - grid envs and one terminal ticket per CTA), so the counters are never reset: the host passes the
- * value a counter has before the launch. */
+ * each launch has its own ticket counter in a ring of BGW_TICKET_RING > resident CTAs.  A launch draws exactly
+ * n_tickets + grid tickets (one terminal ticket per CTA), so the counters are never reset: the host passes the value a
+ * counter has before the launch.
+ * Inside a launch a ticket is a BLOCK of S consecutive manager steps of one env (fast_block_steps): between two steps of
+ * the block the env stays on its CTA with its rows, summary grid and occupant lists in shared memory, and only the
+ * block's first step waits for a stamp (the one the env's previous block -- a smaller ticket, or the launch before --
+ * leaves at its last step).  A CTA still blocks only for the env of its current ticket, whose awaited block has a smaller
+ * ticket number than every ticket its own holder has not finished: the argument above holds for blocks as for steps. */
 #define BGW_TICKET_RING 2048
 __device__ __forceinline__ uint32_t ld_acquire_u32(const uint32_t *p)
 {
@@ -318,6 +325,7 @@ __device__ __forceinline__ void env_wait_stamp(const FastSpec &f, int e, uint32_
     }
 }
 #define BGW_TSLOT 12          /* wsum[12], wsum[13]: the env after this one / the one after that */
+#define BGW_EFSLOT 14         /* wsum[14]: the env flags this step leaves, for the env's next step in the same block */
 
 /* stream env e's rows into one staging buffer */
 __device__ __forceinline__ void fast_issue_env(const DevSpec &s, const FastSpec &f, const BgwState &st, const uint32_t *actions,
@@ -922,19 +930,22 @@ inline bool fast_shape_matches(const DevSpec &q, const FastSpec &f, int threads)
 /* ---- phases of the per-env step (bgw_step_fast_body below), each run by every thread of the CTA ---------------------- */
 
 /* Occupant lists and summary of the relevant entities.  Entry: compaction.  Exit: head / cenc describe the grid, rflag and
- * killrank of the relevant entities are clear (barrier). */
+ * killrank of the relevant entities are clear (barrier).  `kept`: head / cenc still describe the grid from the env's step
+ * before on this CTA (moves and kills keep them exact); only rflag / killrank are cleared, which nothing reads before the
+ * attack pre-pass has ended with its barrier. */
 template <typename HT>
-__device__ __forceinline__ void fast_build_lists(const DevSpec &s, const FastSpec &f, Env &ev, FastEnv &fe, int n_rel, int tid, int T)
+__device__ __forceinline__ void fast_build_lists(const DevSpec &s, const FastSpec &f, Env &ev, FastEnv &fe, int n_rel, bool kept, int tid, int T)
 {
     for (int x = tid; x < n_rel; x += T) {
         const int a = fe.rel[x];
         fe.rflag[a] = 0;
         fe.killrank[a] = BGW_NONE16;
-        if (ev.flags[a] & BGW_ST_IN_GRID) {
+        if (!kept && (ev.flags[a] & BGW_ST_IN_GRID)) {
             if (ev.next[a] != BGW_NONE16) ev.tmp[ev.next[a]] = 1;
             fe.cenc[pad_index(s, f, ev.cell[a])] = ev.enc[a];
         }
     }
+    if (kept) return;
     __syncthreads();
     for (int x = tid; x < n_rel; x += T) {
         const int a = fe.rel[x];
@@ -1111,7 +1122,7 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
             ev.enc[a] = __ldg(&s.enc[a]); ev.klass[a] = k;
         }
     }
-    /* Tickets: ticket g = manager step g / E of env g % E, g < NT.  A CTA draws all its tickets from the launch's counter
+    /* Tickets: ticket g = block g / E (steps [b S, min((b + 1) S, K))) of env g % E, g < NT.  A CTA draws all its tickets from the launch's counter
      * (arrival order); without a counter (a launch captured into a CUDA graph: one step) CTA c takes c, c + grid, ... */
     uint32_t *const tk = f_in.ticket;                      /* this launch's ticket counter */
     const uint32_t NT = f_in.n_tickets, tbase = f_in.ticket_base;
@@ -1141,8 +1152,10 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
     if (!f_in.chain) asm volatile("griddepcontrol.wait;" ::: "memory");
 
     /* (fast_init_dense ended with a barrier: the tickets are visible) */
+    const uint32_t S = f_in.block_steps, K = f_in.n_steps;
     uint32_t g = (uint32_t)tslot[0], gn = 0;
-    int e = 0, kstep = 0, b = 0;
+    int e = 0, kstep = 0, kend = 0, b = 0;                /* this step, the end of its block (exclusive), the staging buffer */
+    bool cont = false;                                     /* not the block's first step: the env's rows are staged in buffer b */
     uint8_t ef_cur = 0, ef_nxt = 0;
     uint32_t step_cur = 0, step_nxt = 0, epi_cur = 0, epi_nxt = 0;
     /* An env's rows may be read once the manager step before has stamped it.  A CTA only ever BLOCKS for the env of its
@@ -1151,10 +1164,10 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
      * ticket (prefetch) a thread merely looks; if the stamp is not there yet it fetches its share of the rows when the
      * ticket becomes current (`late`, per thread: cp.async groups are per thread). */
     bool late = false;
-    int kn_carry = 0, en_carry = 0;
+    int kn_carry = 0, en_carry = 0, kend_carry = 0;
     if (g < NT) {
-        kstep = (int)(g / (uint32_t)s.E); e = (int)(g - (uint32_t)kstep * (uint32_t)s.E);
-        kn_carry = kstep; en_carry = e;
+        const uint32_t blk = g / (uint32_t)s.E;
+        e = (int)(g - blk * (uint32_t)s.E); kstep = (int)(blk * S); kend = (int)min(blk * S + S, K);
         if (f_in.chain || kstep > 0) env_wait_stamp(f_in, e, f_in.seq + (uint32_t)kstep - 1u);
         fast_issue_env(s, f, st, actions, e, bgw_smem + f.o_buf, tid, T);
         ef_cur = __ldcg(&st.env_flags[e]); step_cur = __ldcg(&st.step[e]); epi_cur = __ldcg(&st.episode[e]);
@@ -1163,22 +1176,31 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
 
     uint32_t epoch = f_in.epoch0;                         /* tag of the next reservation round (ordered rounds, above) */
     int it_no = -1, sl = 1;
-    /* end of an env: hand the ticket drawn at its start to the next iteration, and once every thread's stores are
-     * behind a barrier, stamp the env (release: the barrier makes the other threads' stores cumulative).  Thread T - 1
-     * stamps: the fence of the release stalls its warp until the env's stores are performed, so the stamp is on the LAST
-     * warp, not on the warp that leads the env (measured: five episodes 0.0295 -> 0.0276 ms per step). */
+    /* end of an env-step.  Inside a block: the env's flags (written by thread 0 next to st.env_flags), step and episode
+     * carry over to its next step.  At the block's end: hand the ticket drawn at its last step to the next iteration, and
+     * once every thread's stores are behind a barrier, stamp the env (release: the barrier makes the other threads' stores
+     * cumulative).  Thread T - 1 stamps: the fence of the release stalls its warp until the env's stores are performed, so
+     * the stamp is on the LAST warp, not on the warp that leads the env (measured: five episodes 0.0295 -> 0.0276 ms per
+     * step). */
 #define BGW_END_ENV()                                                                \
     do {                                                                             \
-        if (tid == 0) tslot[sl ^ 1] = (int)tnew;                                     \
+        if (tid == 0 && last) tslot[sl ^ 1] = (int)tnew;                             \
         __syncthreads();                                                             \
-        BGW_JITTER_POINT(7);                                                         \
-        if (tid == T - 1) st_release_u32(f_in.env_seq + e, f_in.seq + (uint32_t)kstep); \
-        sl ^= 1;                                                                     \
+        if (last) {                                                                  \
+            BGW_JITTER_POINT(7);                                                     \
+            if (tid == T - 1) st_release_u32(f_in.env_seq + e, f_in.seq + (uint32_t)kstep); \
+            sl ^= 1; b ^= 1; g = gn; cont = false;                                   \
+            kstep = kn_carry; kend = kend_carry; e = en_carry;                       \
+            ef_cur = ef_nxt; step_cur = step_nxt; epi_cur = epi_nxt;                 \
+        } else {                                                                     \
+            ++kstep; cont = true;                                                    \
+            ef_cur = (uint8_t)fe.wsum[BGW_EFSLOT]; step_cur = ev.step; epi_cur = ev.episode; \
+        }                                                                            \
     } while (0)
-    for (; g < NT; g = gn) {
+    while (g < NT) {
         ++it_no;
         BGW_PROF_MARK(0);
-        kstep = kn_carry; e = en_carry;                             /* (step, env) of this ticket: computed when it was `next` */
+        const bool last = kstep + 1 == kend;                       /* the block's last step: the env leaves the CTA after it */
         if (late) {                                                 /* this ticket's rows were not ready when it was `next` */
             env_wait_stamp(f_in, e, f_in.seq + (uint32_t)kstep - 1u);
             fast_issue_env(s, f, st, actions, e, bgw_smem + f.o_buf + b * f.buf_bytes, tid, T);
@@ -1186,28 +1208,32 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
             cp_async_commit();
             late = false;
         }
-        gn = (uint32_t)tslot[sl];
-        uint32_t tnew = NT;                                         /* the ticket after `gn`: drawn now, needed next iteration */
-        BGW_JITTER_POINT(8);
-        if (tid == 0 && gn < NT) tnew = min(NT, tk ? atomicAdd(tk, 1u) - tbase : gn + gridDim.x);
-        if (gn < NT) {
-            const int kn = (int)(gn / (uint32_t)s.E), en = (int)(gn - (uint32_t)kn * (uint32_t)s.E);
-            kn_carry = kn; en_carry = en;
-            if ((f_in.chain || kn > 0) && !env_stamped(f_in, en, f_in.seq + (uint32_t)kn - 1u)) late = true;
-            else {
-                fast_issue_env(s, f, st, actions, en, bgw_smem + f.o_buf + (b ^ 1) * f.buf_bytes, tid, T);
-                ef_nxt = __ldcg(&st.env_flags[en]); step_nxt = __ldcg(&st.step[en]); epi_nxt = __ldcg(&st.episode[en]);
+        uint32_t tnew = NT;                                         /* the ticket after `gn`: drawn now, needed after the next block */
+        if (last) {                                                 /* look at the next ticket as late as possible */
+            gn = (uint32_t)tslot[sl];
+            BGW_JITTER_POINT(8);
+            if (tid == 0 && gn < NT) tnew = min(NT, tk ? atomicAdd(tk, 1u) - tbase : gn + gridDim.x);
+            if (gn < NT) {
+                const uint32_t bn = gn / (uint32_t)s.E;
+                const int kn = (int)(bn * S), en = (int)(gn - bn * (uint32_t)s.E);
+                kn_carry = kn; en_carry = en; kend_carry = (int)min(bn * S + S, K);
+                if ((f_in.chain || kn > 0) && !env_stamped(f_in, en, f_in.seq + (uint32_t)kn - 1u)) late = true;
+                else {
+                    fast_issue_env(s, f, st, actions, en, bgw_smem + f.o_buf + (b ^ 1) * f.buf_bytes, tid, T);
+                    ef_nxt = __ldcg(&st.env_flags[en]); step_nxt = __ldcg(&st.step[en]); epi_nxt = __ldcg(&st.episode[en]);
+                }
             }
         }
-        cp_async_commit();
+        cp_async_commit();                                          /* (an empty group inside a block: wait<1> below stays exact) */
 
         unsigned char *buf = bgw_smem + f.o_buf + b * f.buf_bytes;
         ev.cell = (uint16_t *)(buf + f.b_cell);
         ev.next = (uint16_t *)(buf + f.b_next);
         ev.flags = buf + f.b_flags;
         ev.health = st.health + (size_t)e * s.A;
-        for (int i = tid; i < (s.A * 8 + 127) / 128; i += T)       /* hits read health from HBM on demand: warm L2 now */
-            asm volatile("prefetch.global.L2 [%0];" ::"l"((const char *)ev.health + (size_t)i * 128));
+        if (!cont)
+            for (int i = tid; i < (s.A * 8 + 127) / 128; i += T)   /* hits read health from HBM on demand: warm L2 now */
+                asm volatile("prefetch.global.L2 [%0];" ::"l"((const char *)ev.health + (size_t)i * 128));
         ev.e = e; ev.genv = (uint32_t)(s.env_offset + e);
         int8_t *obs_env = obs ? obs + (size_t)e * s.L * s.obs_stride : nullptr;
         float *rew = reward + (size_t)e * s.L;
@@ -1216,7 +1242,11 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
         const uint8_t ef0 = ef_cur;
         ev.episode = epi_cur;
         ev.step = step_cur + 1u;
-        b ^= 1; ef_cur = ef_nxt; step_cur = step_nxt; epi_cur = epi_nxt;
+        /* the env's next step runs on this CTA from the rows in shared memory (hold), and from this step's summary grid and
+         * occupant lists (hold_lists).  Without auto-reset an env that ends takes no further steps that would store its rows or
+         * clear the summary, so those sims store and clear every step; with mixed cells the lists are rebuilt every step
+         * (ctr[CTR_MIXED] is set only by the rebuild and by the moves). */
+        const bool hold = !last && s.auto_reset, hold_lists = hold && !f.can_mix;
 
         /* rows of learners that receive nothing this call read as zero; zero counters */
         if ((s.L & 15) == 0) {
@@ -1239,7 +1269,7 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
         bool fresh = false;                                         /* this call resets the env instead of stepping it */
         if (__builtin_expect((ef0 & BGW_ENV_ALL_DONE) != 0, 0)) {     /* cold: once per episode */
             if (!s.auto_reset) {
-                if (tid == 0) all_done[e] = ef0;
+                if (tid == 0) { all_done[e] = ef0; fe.wsum[BGW_EFSLOT] = ef0; }
                 BGW_END_ENV();
                 continue;
             }
@@ -1262,7 +1292,7 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
             if (tid == 0) {
                 const uint8_t fl = (uint8_t)((bad ? BGW_ENV_ERROR | BGW_ENV_ALL_DONE : 0) | BGW_ENV_RESET);
                 st.error[e] = (uint32_t)ev.ctr[CTR_ERR];
-                st.env_flags[e] = fl; all_done[e] = fl;
+                st.env_flags[e] = fl; all_done[e] = fl; fe.wsum[BGW_EFSLOT] = fl;
             }
             __syncthreads();
             fast_init_dense(s, f, ev, fe, tid, T);                  /* the reset arena ran over summary and slots */
@@ -1385,7 +1415,7 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
         }
         BGW_PROF_MARK(3);
 
-        fast_build_lists<HT>(s, f, ev, fe, n_rel, tid, T);
+        fast_build_lists<HT>(s, f, ev, fe, n_rel, cont && !fresh && s.auto_reset && !f.can_mix, tid, T);   /* (the step before held them) */
         BGW_PROF_MARK(4);
 
         if (fresh) {
@@ -1486,14 +1516,16 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
             for (int x = tid; x < n_rel; x += T) {
                 const int a = fe.rel[x];
                 const uint8_t fl = ev.flags[a];
-                if (!fresh) { st.cell[off + a] = ev.cell[a]; st.next[off + a] = ev.next[a]; st.flags[off + a] = fl; }
+                /* held rows are stored at the block's end, except those of an entity that leaves the relevant set now (dead,
+                 * removed and reported: the compaction's test), which no later step of the block visits */
+                if (!fresh && (!hold || (fl & 7) == BGW_ST_DONE_REPORTED)) { st.cell[off + a] = ev.cell[a]; st.next[off + a] = ev.next[a]; st.flags[off + a] = fl; }
                 if (fl & BGW_ST_ACTIVE) { const int en2 = ev.enc[a]; if (en2 < 32) lo |= 1u << en2; else hi |= 1u << (en2 - 32); }
                 if (s.done_mask & (BGW_DONE_TARGET_AGENT | BGW_DONE_TARGET_DESTROYED)) {
                     const int t = __ldg(&s.target[a]);
                     if ((s.done_mask & BGW_DONE_TARGET_AGENT) && t >= 0 && !same_position(ev, a, t)) ok = 0;
                     if ((s.done_mask & BGW_DONE_TARGET_DESTROYED) && t >= 0 && (ev.flags[t] & BGW_ST_ACTIVE)) ok = 0;
                 }
-                if (fl & BGW_ST_IN_GRID) fe.cenc[pad_index(s, f, ev.cell[a])] = 0;
+                if ((fl & BGW_ST_IN_GRID) && !hold_lists) fe.cenc[pad_index(s, f, ev.cell[a])] = 0;
             }
             lo = __reduce_or_sync(0xFFFFFFFFu, lo);
             hi = __reduce_or_sync(0xFFFFFFFFu, hi);
@@ -1516,6 +1548,7 @@ __device__ __forceinline__ void bgw_step_fast_body(const DevSpec &s_in, const Fa
             st.step[e] = ev.step;
             st.env_flags[e] = ef;
             all_done[e] = ef;
+            fe.wsum[BGW_EFSLOT] = ef;
             unsigned long long *sr = (unsigned long long *)st.stats + (size_t)e * BGW_STAT_COUNT;
             /* reductions without a return value (the row belongs to this env: no contention): thread 0, which every
              * other thread of the CTA is about to wait for, does not sit out an L2 round trip */
