@@ -1235,7 +1235,9 @@ static __device__ void sim_reset(const DevSpec &s, const BgwState &st, Env &ev, 
     ev.step = 0;
     __syncthreads();                       /* every thread has read episode[e] */
     if (tid == 0) { st.episode[e] = ev.episode; st.step[e] = 0; ev.ctr[CTR_ERR] = 0; }
-    for (int a = tid; a < s.A; a += T) { ev.enc[a] = __ldg(&s.enc[a]); ev.klass[a] = __ldg(&s.klass[a]); ev.racc[a] = 0.0; }
+    /* (the reward accumulators are zeroed at the end: until then their storage is the placement draws' scratch, which
+     * threads other than an accumulator's own write without a barrier in between) */
+    for (int a = tid; a < s.A; a += T) { ev.enc[a] = __ldg(&s.enc[a]); ev.klass[a] = __ldg(&s.klass[a]); }
 
     if (st.layout) {
         /* externally generated placement (MazePlacementState run host-side, state.py:487-527) */

@@ -17,7 +17,9 @@ LIB = os.path.join(ROOT, 'abmarl_b200', 'csrc', 'libbgw_jitter.so')
 def test_parity_under_the_jitter_build():
     env = dict(os.environ, BGW_LIB=LIB)
     sel = 'rollout or chained or full_size or step_sampled or cuda_graph or tb_c5 or tb_c2 or tb_dense or aliased or epochs'
-    r = subprocess.run([sys.executable, '-m', 'pytest', os.path.join(ROOT, 'tests', 'test_gpu_parity.py'), '-x', '-q', '-k', sel],
-                       env=env, cwd=ROOT, capture_output=True, text=True, timeout=1200)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
-    assert ' passed' in r.stdout
+    # the structured policies: long reservation rounds and long occupant lists (the general kernel has no jitter points)
+    for path, k in (('test_gpu_parity.py', sel), ('test_gpu_policies.py', 'not general')):
+        r = subprocess.run([sys.executable, '-m', 'pytest', os.path.join(ROOT, 'tests', path), '-x', '-q', '-k', k],
+                           env=env, cwd=ROOT, capture_output=True, text=True, timeout=1200)
+        assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
+        assert ' passed' in r.stdout

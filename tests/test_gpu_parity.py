@@ -156,6 +156,34 @@ def test_specialized_team_battle_shape_matches_oracle(mirror, name, tmp_path):
     assert_state_equal(eng.state_numpy(), ora.state, name + '/specialized shape, rollout')
 
 
+@pytest.mark.parametrize('name,n_envs,kernel', [('tb_c5_shuffled', 1000, 'stock'), ('tb_c5_shuffled', 1000, 'specialized'),
+                                                ('tb_c5_256_shuffled', 300, 'stock'), ('tb_c5_shuffled', 1000, 'general')])
+def test_shuffled_placement_over_thousands_of_resets(mirror, name, n_envs, kernel, tmp_path, monkeypatch):
+    """PositionState(randomize_placement_order): sim_reset draws the keyed placement order into the storage of the reward
+    accumulators, and a thread that zeroed its accumulator after another thread had drawn there (no barrier between the
+    two) reordered the placement, so the first observations and cells of an occasional episode differed from the
+    reference's.  Horizon 1: every second call resets every env -- bgw_reset, auto-resets in the step kernel (one CTA of
+    three warps per env), in chained rollouts and in the general kernel -- and each is compared with the oracle."""
+    if kernel == 'general':
+        monkeypatch.setenv('BGW_GENERIC_KERNEL', '1')
+    if name == 'tb_c5_256_shuffled':          # the headline shape, two warps in bgw_reset's kernel
+        spec = compile_sim(scenarios.build_tb_c5(mirror), n_envs=n_envs, env_offset=5, seed=0x5EED, horizon=1, auto_reset=True)
+        spec.randomize_placement_order = 1
+    else:
+        builder, manager, _ = scenarios.SCENARIOS[name]
+        spec = compile_sim(builder(mirror), manager=manager, n_envs=n_envs, env_offset=5, seed=0x5EED, horizon=1, auto_reset=True)
+    eng, ora = _pair(spec)
+    if kernel == 'specialized':
+        eng.specialize(cache_dir=str(tmp_path))
+    run_lockstep(eng, ora, 8, label=f'{name}/{kernel} shuffled resets')
+    eng.rollout_sampled(11)
+    for _ in range(11):
+        ora.step(ora.sample_actions())
+    assert_outputs_equal(eng, ora, f'{name}/{kernel} shuffled resets, rollout')
+    assert_state_equal(eng.state_numpy(), ora.state, f'{name}/{kernel} shuffled resets, rollout')
+    assert (ora.state['episode'] >= 9).all()
+
+
 def test_specialize_recompiles_over_a_damaged_cache_entry(mirror, tmp_path):
     """A cache file that does not load (truncated, or from another build) is replaced by a fresh compilation."""
     builder, manager, _ = scenarios.SCENARIOS['traffic']
